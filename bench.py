@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the recurrent off-policy update hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one complete SAC update (`train_one_batch`: sample -> target Q -> critic step + Polyak ->
 actor step -> alpha step; 5 encoder forwards, 2 backwards) with the smamba_s32_c16_b2_nln encoder on a
@@ -26,6 +26,7 @@ Metric: trajectory-steps/s = valid transitions updated on per second, whole job.
 same widths; on CPU its smamba layer walks `Mamba.step` once per time step) on a bounded sample: every trajectory is
 cut to RORL_REF_TLEN (default 100) of its 1000 steps -- the per-step Python loop is linear in the trajectory length,
 so steps/s of the sample is steps/s of the workload, while the row count (what the loop amortises over) is the real 32.
+`--dump-outputs DIR` writes what the last timed update of the `value` arm computed as .npy files (see `dump_outputs`).
 """
 import argparse
 import json
@@ -172,7 +173,12 @@ def run_ours(args):
         return float(ms.item())
 
     # ---- device-resident arm -------------------------------------------------------------------------------------
-    step_dev = lambda: alg.train_one_batch(sync=False)
+    last = [None]
+
+    def step_dev():
+        last[0] = alg.train_one_batch(sync=False)
+        return last[0]
+
     for _ in range(args.warmup):
         out = step_dev()
     valid_steps = out["real_batch_size"]
@@ -183,6 +189,8 @@ def run_ours(args):
     ms_total = timed(step_dev, args.steps)
     launches = NV.launch_count() - l0
     clk = clocks.summary() if clocks else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(alg, last[0], args.dump_outputs)
     ms_per_step = ms_total / args.steps
     value = valid_steps * world / (ms_per_step * 1e-3)
 
@@ -243,6 +251,37 @@ def run_ours(args):
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 63 << 20          # parameters + gradients; the small arrays stay well inside 64 MB in all
+
+
+def dump_outputs(alg, out, path):
+    """`--dump-outputs`: write what the last timed update computed as `path/<name>.npy` -- what `train_one_batch(sync=False)`
+    returned (the device statistics vector and the host scalars) and the state it left: every parameter of the policy,
+    critic and target critic and the gradients of the policy and critic (each model flattened in state_dict order), the
+    entropy temperature and the Q-target guard.  The inputs are seeded, so two builds run with the same arguments can be
+    compared array by array.  Should the parameters and gradients exceed DUMP_BYTES, every one of those arrays keeps
+    every stride-th entry (the same fixed stride for all)."""
+    import torch
+
+    def flat(tensors):
+        return torch.cat([t.detach().reshape(-1).float() for t in tensors]).cpu().numpy()
+
+    arrays = {"stats_device": out["stats_device"].detach().cpu().numpy()}
+    for k in ("real_batch_size", "real_batch_traj_num", "policy_updated"):
+        arrays[k] = np.array(out[k], dtype=np.float64)
+    for name, model in (("policy", alg.policy), ("value", alg.values[0]), ("target_value", alg.target_values[0])):
+        arrays[f"{name}_params"] = flat(t for sd in model.state_dict().values() for t in sd.values())
+    for name, model in (("policy", alg.policy), ("value", alg.values[0])):
+        arrays[f"{name}_grads"] = flat(p.grad for m in model.contextual_modules.values() for p in m.parameters() if p.grad is not None)
+    arrays["log_alpha"] = alg.log_sac_alpha.detach().cpu().numpy()
+    arrays["q_guard"] = alg.Q_guard.state.detach().cpu().numpy()
+    large = [k for k in arrays if k.endswith(("_params", "_grads"))]
+    stride = -(-sum(arrays[k].nbytes for k in large) // DUMP_BYTES)
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a[::stride] if k in large else a)
 
 
 def scan_roofline(alg, dev, ms_per_step):
@@ -508,7 +547,13 @@ if __name__ == "__main__":
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-strong", action="store_true", help="skip the 256-trajectory strong-scaling leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed update computed to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps is not None and a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if a.impl == "reference":
         a.steps = a.steps if a.steps is not None else 3
         a.warmup = a.warmup if a.warmup is not None else 1

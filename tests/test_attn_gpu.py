@@ -50,32 +50,39 @@ def test_attention_vs_oracle(lens, gaps):
         assert_close(x.grad[:, i], ref_in.grad[:, i], TOL, f"d{name}")
 
 
-def test_attention_vs_flash_attn():
-    """Pins the third-party arithmetic: flash-attn's own varlen kernel (bf16) on the same inputs."""
-    fa = pytest.importorskip("flash_attn")
-    import rorl_b200.kernels as K
-    from oracle import attention as OA
-    H, hd = 8, 64
-    lens = [1, 1001, 1, 700, 301]
-    starts, T = _seqs(lens, [0] * len(lens))
+FLASH_LENS, FLASH_H, FLASH_HD = [1, 1001, 1, 700, 301], 8, 64
+FLASH_PROBE = 4099          # stride of the input entries the fixture records, to confirm the inputs are regenerated exactly
+
+
+def flash_attn_case():
+    """Inputs of the flash-attn comparison (CPU): sequence starts, packed qkv [T, 3, H, hd], output gradient [T, H * hd]."""
+    starts, T = _seqs(FLASH_LENS, [0] * len(FLASH_LENS))
     gen = torch.Generator().manual_seed(3)
-    qkv = torch.randn(T, 3, H, hd, generator=gen).cuda()
-    dout = torch.randn(T, H * hd, generator=gen).cuda()
-    slopes = torch.tensor(OA.alibi_slopes(H), dtype=torch.float32, device="cuda")
-    scale = 1.0 / math.sqrt(hd)
-    cu = torch.tensor(np.concatenate(([0], np.cumsum(lens))), dtype=torch.int32, device="cuda")
-    a = qkv.to(torch.bfloat16).requires_grad_()
-    try:
-        ref = fa.flash_attn_varlen_qkvpacked_func(a, cu, max(lens), 0.0, softmax_scale=scale, causal=True, alibi_slopes=slopes)
-    except Exception as e:  # pragma: no cover - flash-attn build without this GPU's kernels
-        pytest.skip(f"flash-attn cannot run here: {e}")
-    ref.backward(dout.view(T, H, hd).to(torch.bfloat16))
-    x = qkv.clone().requires_grad_()
-    tiles, gmap = (t.cuda() for t in K.attention_tiles(starts, lens))
-    out = K.attn_varlen_alibi(x, tiles, gmap, slopes, scale)
-    out.backward(dout)
-    assert_close(out, ref.float().reshape(T, H * hd), 2e-2, "out vs flash-attn (both bf16)")
-    assert_close(x.grad, a.grad.float(), 3e-2, "dqkv vs flash-attn (both bf16)")
+    qkv = torch.randn(T, 3, FLASH_H, FLASH_HD, generator=gen)
+    dout = torch.randn(T, FLASH_H * FLASH_HD, generator=gen)
+    return starts, qkv, dout
+
+
+def test_attention_vs_flash_attn():
+    """Pins the third-party arithmetic: flash-attn 2's own varlen kernel (bf16, ALiBi, causal) on the same inputs, as
+    recorded on a B200 by tests/golden/make_golden_flash_attn.py (attn_flash_varlen.npz: its output and qkv gradient
+    on a fixed, seeded sample of token rows that includes the first and last row of every sequence)."""
+    import rorl_b200.kernels as K
+    from helpers import load_npz
+    from oracle import attention as OA
+    g = load_npz("attn_flash_varlen.npz")
+    starts, qkv, dout = flash_attn_case()
+    assert np.array_equal(qkv.reshape(-1)[::FLASH_PROBE].numpy(), g["qkv_probe"])
+    assert np.array_equal(dout.reshape(-1)[::FLASH_PROBE].numpy(), g["dout_probe"])
+    slopes = torch.tensor(OA.alibi_slopes(FLASH_H), dtype=torch.float32, device="cuda")
+    x = qkv.cuda().requires_grad_()
+    tiles, gmap = (t.cuda() for t in K.attention_tiles(starts, FLASH_LENS))
+    out = K.attn_varlen_alibi(x, tiles, gmap, slopes, 1.0 / math.sqrt(FLASH_HD))
+    out.backward(dout.cuda())
+    rows = torch.from_numpy(g["rows"])
+    bf16 = lambda bits: torch.from_numpy(bits.view(np.int16)).view(torch.bfloat16).float()    # stored as raw bf16 bits
+    assert_close(out.detach().cpu()[rows], bf16(g["out_bf16"]), 2e-2, "out vs flash-attn (both bf16)")
+    assert_close(x.grad.cpu()[rows], bf16(g["dqkv_bf16"]), 3e-2, "dqkv vs flash-attn (both bf16)")
 
 
 @pytest.mark.parametrize("case", ["stacked_ln", "rows_rms"])
