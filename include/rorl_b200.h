@@ -308,6 +308,28 @@ int rorl_gru_bwd(const float* dout, const float* dh_last, const float* w_hh, con
                  cudaStream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * LSTM recurrence as a persistent thread-block-cluster kernel (W_hh resident in registers across a
+ * cluster of H / 32 CTAs, h_t exchanged through distributed shared memory each step; csrc/lstm.cu).
+ * Replaces the recurrent part of torch.nn.LSTM(input, H, batch_first=True) on the `lstm` encoder path
+ * (ref: offpolicy_rnn/models/rnn_base.py layer table 'lstm' -> nn.LSTM; gate order i, f, g, o as in torch.nn.LSTM:
+ * gates = gi + h W_hh^T + b_hh, c' = sigmoid(f) c + sigmoid(i) tanh(g), h' = sigmoid(o) tanh(c')).
+ * gi [B, L, 4H] = x W_ih^T + b_ih is computed by the caller (one GEMM); w_hh [4H, H] (16-byte aligned); b_hh [4H]
+ * or NULL; h0, c0 [B, H] or NULL (= 0).  out [B, L, H] = h_t for every step; h_last, c_last [B, H] (may be NULL);
+ * save [B, L, 5H] = (sigmoid(i), sigmoid(f), tanh(g), sigmoid(o), c_t) per step for the backward (NULL when no
+ * backward follows; rorl_lstm_save_floats_per_step(H) = 5H).  H in {16, 32, 64, 128, 256}.
+ * Backward: dout [B, L, H] (gradient w.r.t. out), dh_last, dc_last [B, H] or NULL (= 0), the forward's save and c0
+ * -> dgates [B, L, 4H] (gradient w.r.t. the pre-activation gates = w.r.t. gi = w.r.t. b_hh per step), dh0, dc0
+ * [B, H] (may be NULL).  Weight gradients are GEMMs over all steps, left to the caller: dW_hh = dgates^T h_{t-1}.
+ * Deterministic (no atomics), no host synchronisation or allocation: both launches can be graph-captured.
+ * ---------------------------------------------------------------------------------------------- */
+int rorl_lstm_save_floats_per_step(int64_t H);
+int rorl_lstm_fwd(const float* gi, const float* w_hh, const float* b_hh, const float* h0, const float* c0, float* out,
+                  float* save, float* h_last, float* c_last, int64_t B, int64_t L, int64_t H, cudaStream_t stream);
+int rorl_lstm_bwd(const float* dout, const float* dh_last, const float* dc_last, const float* w_hh, const float* save,
+                  const float* c0, float* dgates, float* dh0, float* dc0, int64_t B, int64_t L, int64_t H,
+                  cudaStream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Causal variable-length attention with ALiBi on tcgen05 tensor cores (bf16 operands, fp32 accumulate), head
  * dimension 64.  Replaces flash_attn_varlen_qkvpacked_func(qkv[T, 3, H, 64], cu_seqlens, max_seqlen, p = 0,
  * softmax_scale, causal = True, alibi_slopes) as used by flash_attn's MHA in the cgpt encoder layer

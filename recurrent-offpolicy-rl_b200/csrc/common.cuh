@@ -114,4 +114,35 @@ __device__ __forceinline__ float warp_min(float v) {
     return v;
 }
 
+// ---- persistent thread-block-cluster recurrences (csrc/gru.cu, csrc/lstm.cu) ----
+// Launch a 1-D grid of nclusters clusters of cl CTAs each; returns RORL_OK or 1000 + cudaError_t.
+template <typename Kern, typename Params>
+static int launch_cluster(Kern kern, const Params& p, int cl, int nthreads, int nclusters, cudaStream_t stream) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)(cl * nclusters));
+    cfg.blockDim = dim3((unsigned)nthreads);
+    cfg.dynamicSmemBytes = 0;
+    cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = (unsigned)cl;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    cudaError_t e = cudaLaunchKernelEx(&cfg, kern, p);
+    if (e != cudaSuccess) {
+        (void)cudaGetLastError();
+        return 1000 + (int)e;
+    }
+    return RORL_OK;
+}
+
+// batch rows per cluster: smallest power of two that fits the batch into <= max_clusters clusters
+static inline int pick_bg(int64_t B, int max_clusters) {
+    int bg = 1;
+    while (bg < 4 && (B + bg - 1) / bg > max_clusters) bg <<= 1;
+    return bg;
+}
+
 }  // namespace rorl

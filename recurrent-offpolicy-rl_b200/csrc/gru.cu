@@ -265,35 +265,6 @@ __global__ void __launch_bounds__(GruCfg<H>::NT, 1) gru_bwd_kernel(const GruBwdP
     }
 }
 
-template <typename Kern, typename Params>
-static int launch_cluster(Kern kern, const Params& p, int cl, int nthreads, int nclusters, cudaStream_t stream) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(cl * nclusters));
-    cfg.blockDim = dim3((unsigned)nthreads);
-    cfg.dynamicSmemBytes = 0;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = (unsigned)cl;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, kern, p);
-    if (e != cudaSuccess) {
-        (void)cudaGetLastError();
-        return 1000 + (int)e;
-    }
-    return RORL_OK;
-}
-
-// batch rows per cluster: smallest power of two that fits the batch into <= max_clusters clusters
-static int pick_bg(int64_t B, int max_clusters) {
-    int bg = 1;
-    while (bg < 4 && (B + bg - 1) / bg > max_clusters) bg <<= 1;
-    return bg;
-}
-
 }  // namespace rorl
 
 using namespace rorl;

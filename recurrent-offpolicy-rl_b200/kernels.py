@@ -7,6 +7,7 @@ Each Function is the B200 counterpart of one autograd Function / fused op of the
   SelectiveScan / selective_scan_fn     <- SelectiveScanFn (ref: offpolicy_rnn/models/smamba/mamba_ssm/ops/selective_scan_interface_new.py:19-93)
   AddNorm / layer_norm_fn, rms_norm_fn  <- LayerNormFn (ref: offpolicy_rnn/models/smamba/mamba_ssm/ops/triton/layernorm.py:464-478)
   GRUScan                               <- torch.nn.GRU recurrence (ref: offpolicy_rnn/models/rnn_base.py:59,245-247,454)
+  LSTMScan                              <- torch.nn.LSTM recurrence (ref: offpolicy_rnn/models/rnn_base.py layer table 'lstm')
   CausalConv1dSiLU                      <- mask * x -> nn.Conv1d -> SiLU (ref: offpolicy_rnn/models/smamba/mamba.py:207-212)
 
 All of them require CUDA tensors: there is no CPU implementation (the oracle under oracle/ is test
@@ -461,6 +462,66 @@ class GRUScan(Function):
 
 def gru_scan(gi, w_hh, b_hh=None, h0=None):
     return GRUScan.apply(gi, w_hh, b_hh, h0)
+
+
+# ------------------------------------------------------------------------------------------------
+# LSTM (persistent cluster kernel for the recurrence; the input / weight-gradient GEMMs are tensor-core GEMMs)
+# ------------------------------------------------------------------------------------------------
+class LSTMScan(Function):
+    """out, h_last, c_last = LSTM recurrence over gi = x W_ih^T + b_ih.  gi [B, L, 4H]; w_hh [4H, H]; b_hh [4H];
+    h0, c0 [B, H] (any shape with B * H elements, or None = 0).  Gate order i, f, g, o as in torch.nn.LSTM."""
+
+    @staticmethod
+    def forward(ctx, gi, w_hh, b_hh, h0, c0):
+        gi, w = _f32c(gi), _f32c(w_hh)
+        B, L, H4 = gi.shape
+        H = H4 // 4
+        b = None if b_hh is None else _f32c(b_hh)
+        h0c = None if h0 is None else _f32c(h0.reshape(B, H))
+        c0c = None if c0 is None else _f32c(c0.reshape(B, H))
+        dev = gi.device
+        out = torch.empty((B, L, H), device=dev, dtype=torch.float32)
+        h_last = torch.empty((B, H), device=dev, dtype=torch.float32)
+        c_last = torch.empty((B, H), device=dev, dtype=torch.float32)
+        save = (torch.empty((B, L, int(N.lib().rorl_lstm_save_floats_per_step(H))), device=dev, dtype=torch.float32)
+                if any(ctx.needs_input_grad) else None)
+        N.call("rorl_lstm_fwd", N.ptr(gi), N.ptr(w), N.ptr(b), N.ptr(h0c), N.ptr(c0c), N.ptr(out), N.ptr(save),
+               N.ptr(h_last), N.ptr(c_last), B, L, H, N.stream())
+        ctx.save_for_backward(w, save, out, h0c, c0c)
+        ctx.has_bias = b is not None
+        ctx.h0_shape = None if h0 is None else h0.shape
+        ctx.c0_shape = None if c0 is None else c0.shape
+        ctx.set_materialize_grads(False)
+        return out, h_last, c_last
+
+    @staticmethod
+    def backward(ctx, dout, dh_last, dc_last):
+        w, save, out, h0c, c0c = ctx.saved_tensors
+        B, L, H = out.shape
+        dev = out.device
+        dout = torch.zeros_like(out) if dout is None else _f32c(dout)
+        dh_last = None if dh_last is None else _f32c(dh_last.reshape(B, H))
+        dc_last = None if dc_last is None else _f32c(dc_last.reshape(B, H))
+        dgates = torch.empty((B, L, 4 * H), device=dev, dtype=torch.float32)
+        dh0 = torch.empty((B, H), device=dev, dtype=torch.float32)
+        dc0 = torch.empty((B, H), device=dev, dtype=torch.float32)
+        N.call("rorl_lstm_bwd", N.ptr(dout), N.ptr(dh_last), N.ptr(dc_last), N.ptr(w), N.ptr(save), N.ptr(c0c),
+               N.ptr(dgates), N.ptr(dh0), N.ptr(dc0), B, L, H, N.stream())
+        g2 = dgates.view(B * L, 4 * H)
+        dw = db = None
+        if ctx.needs_input_grad[1]:
+            first = torch.zeros((B, 1, H), device=dev, dtype=torch.float32) if h0c is None else h0c.unsqueeze(1)
+            h_prev = torch.cat((first, out[:, :-1]), dim=1).reshape(B * L, H)
+            dw = gemm_nt(g2, h_prev) if _gemm_nt_ok(4 * H, H, B * L) else g2.t() @ h_prev
+        if ctx.has_bias and ctx.needs_input_grad[2]:
+            db = colsum(g2)
+        dh0_out = dh0.view(ctx.h0_shape) if (ctx.h0_shape is not None and ctx.needs_input_grad[3]) else None
+        dc0_out = dc0.view(ctx.c0_shape) if (ctx.c0_shape is not None and ctx.needs_input_grad[4]) else None
+        return dgates, dw, db, dh0_out, dc0_out
+
+
+def lstm_scan(gi, w_hh, b_hh=None, h0=None, c0=None):
+    return LSTMScan.apply(gi, w_hh, b_hh, h0, c0)
 
 
 # ------------------------------------------------------------------------------------------------

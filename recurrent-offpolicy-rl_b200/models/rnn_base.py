@@ -30,6 +30,7 @@ from .s6.mamba import MambaResidualBlock
 from .conv1d.conv1d import Conv1d
 from .gilr_lstm.gilr_lstm import GILRLSTMLayer
 from .gru.gru import GRULayer
+from .lstm.lstm import LSTMLayer
 
 try:
     from .flash_attention.TransformerFlashAttention import TransformerDecoder
@@ -100,7 +101,7 @@ def parse_layer_id(layer_id: str) -> Tuple[str, Dict]:
             else:
                 raise ValueError(f'Pattern {t} has not been implemented!')
         return 'cgpt', cfg
-    if layer_id in ('gru', 'lru', 'gilr', 'gilr_lstm'):
+    if layer_id in ('gru', 'lstm', 'lru', 'gilr', 'gilr_lstm'):
         return layer_id, {}
     if layer_id.startswith('conv1d'):                          # ref: rnn_base.py:227-234
         return 'conv1d', {'d_conv': int(layer_id.split('_')[-1]) if '_' in layer_id else 4}
@@ -117,7 +118,7 @@ def parse_layer_id(layer_id: str) -> Tuple[str, Dict]:
                                   "constructor there (its layer_dict has no such key, ref :55-69): it cannot be built in the reference either")
     raise NotImplementedError(
         f'layer type {layer_id!r} is outside the update hot path this package covers '
-        f'(fc, efc-E, gru, lru, gilr, gilr_lstm, conv1d_*, smamba_*, mamba_*, cgpt_*, elru-E, egilr-E, egilr_lstm-E, econv1d_*-E)')
+        f'(fc, efc-E, gru, lstm, lru, gilr, gilr_lstm, conv1d_*, smamba_*, mamba_*, cgpt_*, elru-E, egilr-E, egilr_lstm-E, econv1d_*-E)')
 
 
 class RNNBase(nn.Module):
@@ -155,6 +156,9 @@ class RNNBase(nn.Module):
                     self.rnn_hidden_state_input_size.append(width)
                 elif kind == 'gru':
                     self.layer_list.append(GRULayer(width_in, width, batch_first=True))
+                    self.rnn_hidden_state_input_size.append(width)
+                elif kind == 'lstm':
+                    self.layer_list.append(LSTMLayer(width_in, width, batch_first=True))
                     self.rnn_hidden_state_input_size.append(width)
                 elif kind == 'gilr_lstm':
                     self.layer_list.append(GILRLSTMLayer(width_in, width, batch_first=True))
@@ -246,7 +250,7 @@ class RNNBase(nn.Module):
                 self._xavier_multi(m.in_proj)
             elif isinstance(m, (MambaBlockList, MambaResidualBlock, Conv1d, EConv1d)) or (TransformerDecoder is not None and isinstance(m, TransformerDecoder)):
                 pass
-            else:   # GRU and anything else with plain weight/bias tensors
+            else:   # GRU, LSTM and anything else with plain weight/bias tensors
                 for name, param in m.named_parameters():
                     if 'weight' in name:
                         nn.init.xavier_uniform_(param.data)
