@@ -331,22 +331,25 @@ int rorl_lstm_bwd(const float* dout, const float* dh_last, const float* dc_last,
 
 /* ------------------------------------------------------------------------------------------------
  * Causal variable-length attention with ALiBi on tcgen05 tensor cores (bf16 operands, fp32 accumulate), head
- * dimension 64.  Replaces flash_attn_varlen_qkvpacked_func(qkv[T, 3, H, 64], cu_seqlens, max_seqlen, p = 0,
+ * dimension hd = any multiple of 8 from 8 to 128 (the _hd entry points; the entry points without the suffix are those
+ * with hd = 64).  Replaces flash_attn_varlen_qkvpacked_func(qkv[T, 3, H, hd], cu_seqlens, max_seqlen, p = 0,
  * softmax_scale, causal = True, alibi_slopes) as used by flash_attn's MHA in the cgpt encoder layer
  * (ref: offpolicy_rnn/models/flash_attention/TransformerFlashAttention.py:65-85,104-121).
  *
  * Token spaces.  TMA needs 16-byte aligned inner coordinates, so inside the attention kernels every sequence starts
  * on an 8-token boundary of an ATTENTION TOKEN SPACE of T tokens (Tp = T rounded up to a multiple of 64); gmap
  * (device int32[T], or NULL = identity) gives the source row of each attention-space token (-1 = padding slot).
- * rorl_attn_prep gathers an fp32 source [rows, nsec, H, 64] (row stride ld_tok floats) into bf16 copies in that
- * space: row-major rm [nsec][T, H, 64] and token-contiguous tr [nsec][H, 64, Tp] (either may be NULL); with
- * o != NULL (nsec == 1, o in SOURCE rows) it also writes D[H, Tp] = sum_d src * o (the backward's row statistic).
- * bf16 buffers are passed as void*.
+ * rorl_attn_prep gathers an fp32 source [rows, nsec, H, hd] (row stride ld_tok floats) into bf16 copies in that
+ * space, padded along d to DP = 64 (hd <= 64) or DP = 128 (hd > 64) with zero columns: row-major rm [nsec][T, H, DP]
+ * and token-contiguous tr [nsec][H, DP, Tp] (either may be NULL); with o != NULL (nsec == 1, o [rows, H, hd] in
+ * SOURCE rows, row stride ld_o) it also writes D[H, Tp] = sum_d src * o (the backward's row statistic).
+ * bf16 buffers are passed as void*.  The forward and backward take these DP-padded copies.
  * tiles: device int32[ntiles][4] = (first attention-space token of the sequence, sequence length, 128-row tile
  * index, first OUTPUT row of the sequence), one entry per 128-row tile of every sequence.
- * Forward: O fp32 with row stride ld_o, written at OUTPUT rows (columns h*64 .. h*64+63 of head h; other rows are
- * not touched), lse [H, Tp] (log2 domain, attention space) for the backward (may be NULL).
- * Backward: dq, dk, dv fp32 with row stride ld_d, written at OUTPUT rows.
+ * Forward: O fp32 with row stride ld_o, written at OUTPUT rows (columns h*hd .. h*hd+hd-1 of head h; other rows
+ * and columns are not touched), lse [H, Tp] (log2 domain, attention space) for the backward (may be NULL).
+ * Backward: dq, dk, dv fp32 with row stride ld_d, written at OUTPUT rows, columns h*hd .. h*hd+hd-1.
+ * An unsupported head_dim returns RORL_ERR_SHAPE.
  * dropout_p > 0: attention-probability dropout (flash-attn's dropout_p; ref TransformerFlashAttention.py:65-70):
  * keep bits come from a counter hash of (seed[0] (device int64), salt, head, query token, key token); the backward
  * must be given the same (dropout_p, seed value, salt) as its forward.  dropout_p == 0: seed may be NULL.
@@ -361,6 +364,17 @@ int rorl_attn_bwd(const void* q_rm, const void* k_rm, const void* v_rm, const vo
                   int64_t ntiles, const float* slopes, float softmax_scale, float* dq, float* dk, float* dv,
                   int64_t ld_d, int64_t H, int64_t T, int64_t Tp, float dropout_p, const int64_t* seed, int64_t salt,
                   cudaStream_t stream);
+int rorl_attn_prep_hd(const float* src, int64_t ld_tok, int64_t nsec, int64_t H, int64_t T, int64_t Tp, const int32_t* gmap,
+                      void* rm_bf16, void* tr_bf16, const float* o, int64_t ld_o, float* Dout, int64_t head_dim,
+                      cudaStream_t stream);
+int rorl_attn_fwd_hd(const void* q_rm, const void* k_rm, const void* v_tr, const int32_t* tiles, int64_t ntiles,
+                     const float* slopes, float softmax_scale, float* O, int64_t ld_o, float* lse, int64_t H, int64_t T,
+                     int64_t Tp, float dropout_p, const int64_t* seed, int64_t salt, int64_t head_dim, cudaStream_t stream);
+int rorl_attn_bwd_hd(const void* q_rm, const void* k_rm, const void* v_rm, const void* do_rm, const void* q_tr,
+                     const void* k_tr, const void* do_tr, const float* lse, const float* D, const int32_t* tiles,
+                     int64_t ntiles, const float* slopes, float softmax_scale, float* dq, float* dk, float* dv,
+                     int64_t ld_d, int64_t H, int64_t T, int64_t Tp, float dropout_p, const int64_t* seed, int64_t salt,
+                     int64_t head_dim, cudaStream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Trajectory gather: builds the padded, nest-stacked [rows, Lmax, F] fp32 batch of

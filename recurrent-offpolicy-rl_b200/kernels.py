@@ -1142,49 +1142,56 @@ def ensemble_linear(x, weight, bias, elu, shared):
 # ------------------------------------------------------------------------------------------------
 # causal variable-length attention with ALiBi (tcgen05, bf16 operands) -- the cgpt encoder's attention
 # ------------------------------------------------------------------------------------------------
+ATTN_HEAD_DIMS = tuple(range(8, 129, 8))          # head dimensions the attention kernels take
+
+
 class AttnVarlen(Function):
-    """out[T, H*64] = attention(qkv[T, 3, H, 64]) per sequence.  `tiles` int32 [ntiles, 4] and `gmap` int32 [Ta] on the
-    device come from attention_tiles (see include/rorl_b200.h for the two token spaces); slopes [H] fp32.
+    """out[T, H*hd] = attention(qkv[T, 3, H, hd]) per sequence, hd in ATTN_HEAD_DIMS.  `tiles` int32 [ntiles, 4] and
+    `gmap` int32 [Ta] on the device come from attention_tiles (see include/rorl_b200.h for the two token spaces); slopes
+    [H] fp32.  The kernels' bf16 operand copies are padded with zeros along d to 64 (hd <= 64) or 128.
     dropout_p > 0: attention-probability dropout with the keep mask hashed from (`seed` device int64 [1], `salt`, head,
     query, key); the backward regenerates the same mask."""
 
     @staticmethod
     def forward(ctx, qkv, tiles, gmap, slopes, softmax_scale, dropout_p=0.0, seed=None, salt=0):
         T, three, H, hd = qkv.shape
-        assert three == 3 and hd == 64, "the tcgen05 attention kernel is built for head dimension 64"
+        if three != 3 or hd not in ATTN_HEAD_DIMS:
+            raise NotImplementedError(f"attention takes qkv [T, 3, H, hd] with hd a multiple of 8 from 8 to 128, got {tuple(qkv.shape)}")
         qkv = _f32c(qkv)
         dev = qkv.device
         Ta = gmap.shape[0]
         Tp = (Ta + 63) // 64 * 64
+        Dp = 64 if hd <= 64 else 128
         need_grad = ctx.needs_input_grad[0]
-        rm = torch.empty((3, Ta, H, 64), device=dev, dtype=torch.bfloat16)
-        tr = torch.empty((3, H, 64, Tp), device=dev, dtype=torch.bfloat16)
-        N.call("rorl_attn_prep", N.ptr(qkv), 3 * H * 64, 3, H, Ta, Tp, N.ptr(gmap), N.ptr(rm), N.ptr(tr), None, 0, None, N.stream())
-        out = torch.zeros((T, H * 64), device=dev, dtype=torch.float32)        # rows outside every sequence stay 0
+        rm = torch.empty((3, Ta, H, Dp), device=dev, dtype=torch.bfloat16)
+        tr = torch.empty((3, H, Dp, Tp), device=dev, dtype=torch.bfloat16)
+        N.call("rorl_attn_prep_hd", N.ptr(qkv), 3 * H * hd, 3, H, Ta, Tp, N.ptr(gmap), N.ptr(rm), N.ptr(tr), None, 0, None, hd,
+               N.stream())
+        out = torch.zeros((T, H * hd), device=dev, dtype=torch.float32)        # rows outside every sequence stay 0
         lse = torch.zeros((H, Tp), device=dev, dtype=torch.float32) if need_grad else None
         dropout_p = float(dropout_p)
-        N.call("rorl_attn_fwd", N.ptr(rm[0]), N.ptr(rm[1]), N.ptr(tr[2]), N.ptr(tiles), tiles.shape[0], N.ptr(slopes),
-               float(softmax_scale), N.ptr(out), H * 64, N.ptr(lse), H, Ta, Tp, dropout_p, N.ptr(seed if dropout_p > 0 else None),
-               int(salt), N.stream())
+        N.call("rorl_attn_fwd_hd", N.ptr(rm[0]), N.ptr(rm[1]), N.ptr(tr[2]), N.ptr(tiles), tiles.shape[0], N.ptr(slopes),
+               float(softmax_scale), N.ptr(out), H * hd, N.ptr(lse), H, Ta, Tp, dropout_p, N.ptr(seed if dropout_p > 0 else None),
+               int(salt), hd, N.stream())
         ctx.save_for_backward(rm, tr, out, lse, tiles, gmap, slopes, seed if dropout_p > 0 else None)
-        ctx.scale, ctx.dims, ctx.drop = float(softmax_scale), (T, H, Ta, Tp), (dropout_p, int(salt))
+        ctx.scale, ctx.dims, ctx.drop = float(softmax_scale), (T, H, hd, Dp, Ta, Tp), (dropout_p, int(salt))
         return out
 
     @staticmethod
     def backward(ctx, dout):
         rm, tr, out, lse, tiles, gmap, slopes, seed = ctx.saved_tensors
-        T, H, Ta, Tp = ctx.dims
+        T, H, hd, Dp, Ta, Tp = ctx.dims
         dev = out.device
         dout = _f32c(dout)
-        do_rm = torch.empty((Ta, H, 64), device=dev, dtype=torch.bfloat16)
-        do_tr = torch.empty((H, 64, Tp), device=dev, dtype=torch.bfloat16)
+        do_rm = torch.empty((Ta, H, Dp), device=dev, dtype=torch.bfloat16)
+        do_tr = torch.empty((H, Dp, Tp), device=dev, dtype=torch.bfloat16)
         D = torch.empty((H, Tp), device=dev, dtype=torch.float32)
-        N.call("rorl_attn_prep", N.ptr(dout), H * 64, 1, H, Ta, Tp, N.ptr(gmap), N.ptr(do_rm), N.ptr(do_tr), N.ptr(out), H * 64,
-               N.ptr(D), N.stream())
-        dqkv = torch.zeros((T, 3, H, 64), device=dev, dtype=torch.float32)
-        N.call("rorl_attn_bwd", N.ptr(rm[0]), N.ptr(rm[1]), N.ptr(rm[2]), N.ptr(do_rm), N.ptr(tr[0]), N.ptr(tr[1]), N.ptr(do_tr),
+        N.call("rorl_attn_prep_hd", N.ptr(dout), H * hd, 1, H, Ta, Tp, N.ptr(gmap), N.ptr(do_rm), N.ptr(do_tr), N.ptr(out), H * hd,
+               N.ptr(D), hd, N.stream())
+        dqkv = torch.zeros((T, 3, H, hd), device=dev, dtype=torch.float32)
+        N.call("rorl_attn_bwd_hd", N.ptr(rm[0]), N.ptr(rm[1]), N.ptr(rm[2]), N.ptr(do_rm), N.ptr(tr[0]), N.ptr(tr[1]), N.ptr(do_tr),
                N.ptr(lse), N.ptr(D), N.ptr(tiles), tiles.shape[0], N.ptr(slopes), ctx.scale, N.ptr(dqkv[:, 0]), N.ptr(dqkv[:, 1]),
-               N.ptr(dqkv[:, 2]), 3 * H * 64, H, Ta, Tp, ctx.drop[0], N.ptr(seed), ctx.drop[1], N.stream())
+               N.ptr(dqkv[:, 2]), 3 * H * hd, H, Ta, Tp, ctx.drop[0], N.ptr(seed), ctx.drop[1], hd, N.stream())
         return dqkv, None, None, None, None, None, None, None
 
 

@@ -71,8 +71,9 @@ class MHA(nn.Module):
         self.layer_idx = layer_idx
         assert embed_dim % num_heads == 0
         self.embed_dim, self.num_heads, self.head_dim = embed_dim, num_heads, embed_dim // num_heads
-        if self.head_dim != 64:
-            raise NotImplementedError('the tcgen05 attention kernel is built for head dimension 64 (cgpt: 512 / 8)')
+        if self.head_dim not in K.ATTN_HEAD_DIMS:
+            raise NotImplementedError(f'the tcgen05 attention kernels take head dimensions 8, 16, ..., 128 (multiples of 8); '
+                                      f'got {self.head_dim} (width {embed_dim} / {num_heads} heads)')
         self.attn_dropout = dropout
         self.Wqkv = Linear(embed_dim, 3 * embed_dim)
         self.out_proj = Linear(embed_dim, embed_dim)
@@ -99,10 +100,11 @@ class MHA(nn.Module):
 
     def decode_step(self, x, cache):
         """One rollout step with the kv-cache: x [B, 1, C]; `cache` is the layer stack's InferenceParams
-        (`key_value_memory_dict[layer_idx]` = [max_batch, max_seqlen, 2, H, 64] bf16, `seqlen_offset` = tokens already
+        (`key_value_memory_dict[layer_idx]` = [max_batch, max_seqlen, 2, H, hd] bf16, `seqlen_offset` = tokens already
         cached).  Same arithmetic as the training kernel on one query row: bf16 q / k / v, fp32 scores with the ALiBi
         bias -slope * (offset - j), fp32 softmax, bf16 probabilities.  (ref: flash_attn MHA with inference_params as
-        called from TransformerFlashAttention.py:76-83 and rnn_base.py:437-452.)  Tiny tensors: plain CUDA ops."""
+        called from TransformerFlashAttention.py:76-83 and rnn_base.py:437-452.)  Tiny tensors: plain CUDA ops, the same
+        for every head dimension hd."""
         B = x.shape[0]
         H, hd = self.num_heads, self.head_dim
         qkv = K.linear(x, self.Wqkv.weight, self.Wqkv.bias, passes=BF16_AUTOCAST_PASSES).view(B, 3, H, hd)

@@ -2,7 +2,7 @@
 """Per-kernel micro-benchmark at the workload shapes (SURVEY.md 8d): CUDA-event time per launch, algorithmic
 bytes / FLOPs, fraction of the measured peak.  Inputs are larger than L2 or rotated so launches do not hit in cache.
 
-    python tools/bench_kernels.py [--only gilr,lru,selscan,conv,addnorm,gru,lstm,gemm] [--out kernels.json]
+    python tools/bench_kernels.py [--only gilr,lru,selscan,conv,addnorm,gru,lstm,gemm,attn,attn_hd] [--out kernels.json]
 """
 import argparse
 import json
@@ -332,6 +332,53 @@ def bench_attn():
         print("flash-attn unavailable:", e)
 
 
+def attn_flops(lens, H, hd):
+    """Algorithmic FLOPs of causal attention over sequences `lens`: Q K^T and P V, 2 * hd each per (query, key <= query)
+    pair.  The backward's five products are counted as 2.5 forwards (forward + backward = 3.5x)."""
+    return sum(4.0 * n * (n + 1) / 2 * hd for n in lens) * H
+
+
+def bench_attn_hd():
+    """cgpt attention at other head dimensions (32 sequences x 1001 tokens; width / heads = hd), next to flash-attn 2's
+    varlen kernel on the same inputs when it imports.  hd <= 64 runs on operands padded to 64, hd > 64 on 128; the
+    FLOP/s below count the real hd only."""
+    import math
+    import numpy as np
+    lens = [1001] * 32
+    starts = [1001 * i for i in range(32)]
+    T = sum(lens)
+    tiles, gmap = (t.to(dev) for t in K.attention_tiles(starts, lens))
+    try:
+        import flash_attn as fa
+    except Exception as e:  # pragma: no cover
+        fa = None
+        print("flash-attn unavailable:", e)
+    cu = torch.tensor(np.concatenate(([0], np.cumsum(lens))), dtype=torch.int32, device=dev)
+    for width, H in ((256, 8), (512, 8), (512, 4), (1024, 8)):
+        hd = width // H
+        qkv = rn(T, 3, H, hd).requires_grad_()
+        dout = rn(T, H * hd)
+        slopes = torch.tensor([2 ** (-(i + 1)) for i in range(H)], dtype=torch.float32, device=dev)
+        scale = 1.0 / math.sqrt(hd)
+        fl_f = attn_flops(lens, H, hd)
+        tag = f"C={width} H={H} hd={hd}"
+        with torch.no_grad():
+            t_f = timeit(lambda: K.attn_varlen_alibi(qkv, tiles, gmap, slopes, scale))
+        t_fb = timeit(lambda: torch.autograd.grad(K.attn_varlen_alibi(qkv, tiles, gmap, slopes, scale), qkv, dout), n=10)
+        rec(f"attn_fwd {tag} (ours: prep + tcgen05 kernel, fp32 in/out)", t_f, flops=fl_f)
+        rec(f"attn_fwd+bwd {tag} (ours)", t_fb, flops=3.5 * fl_f)
+        if fa is not None:
+            a = qkv.detach().to(torch.bfloat16).requires_grad_()
+            do16 = dout.view(T, H, hd).to(torch.bfloat16)
+            call = lambda: fa.flash_attn_varlen_qkvpacked_func(a, cu, max(lens), 0.0, softmax_scale=scale, causal=True, alibi_slopes=slopes)
+            with torch.no_grad():
+                t_f = timeit(call)
+            t_fb = timeit(lambda: torch.autograd.grad(call(), a, do16), n=10)
+            rec(f"flash-attn 2 varlen fwd {tag} (library, same box, bf16 in/out)", t_f, flops=fl_f, note=f"flash_attn {fa.__version__}")
+            rec(f"flash-attn 2 varlen fwd+bwd {tag} (library, same box)", t_fb, flops=3.5 * fl_f)
+        del qkv, dout
+
+
 def bench_refs():
     """The reference's own in-tree Triton scans (K6 / K7) on the same box, imported UNMODIFIED from oracle/_ref
     (ref: gilr/scan_triton/real_rnn_tie_input_gate.py:170-264, lru/scan_triton/complex_rnn.py:174-244)."""
@@ -371,7 +418,7 @@ def bench_refs():
         print("reference lru Triton scan failed:", repr(e))
 
 
-ALL = {"attn": bench_attn, "refs": bench_refs, "reduce": bench_reduce, "gilr": bench_gilr, "lru": bench_lru, "lru_fused": bench_lru_fused, "selscan": bench_selscan, "conv": bench_conv, "addnorm": bench_addnorm,
+ALL = {"attn": bench_attn, "attn_hd": bench_attn_hd, "refs": bench_refs, "reduce": bench_reduce, "gilr": bench_gilr, "lru": bench_lru, "lru_fused": bench_lru_fused, "selscan": bench_selscan, "conv": bench_conv, "addnorm": bench_addnorm,
        "gru": bench_gru, "lstm": bench_lstm, "gemm": bench_gemm}
 
 if __name__ == "__main__":
