@@ -214,31 +214,38 @@ int rorl_adamw_polyak(float* p, float* g, float* m, float* v, float* target, con
 int rorl_sumsq(const float* p, int64_t n, float* out, float* work, cudaStream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
- * tcgen05 tensor-core GEMM with fp32 parity (3xTF32 split accumulation in the TMEM accumulator).
+ * tcgen05 tensor-core GEMM with fp32 parity: every fp32 operand is split into bf16 hi + lo and the product is
+ * accumulated as lo*hi + hi*lo + hi*hi in the fp32 TMEM accumulator.
  * Replaces the cuBLAS fp32 SGEMMs behind nn.Linear / EnsembleLinear (ref: offpolicy_rnn/models/
  * ensemble_linear_model.py:36-49; smamba projections, ref: offpolicy_rnn/models/smamba/mamba.py:176,231-233,252).
  *   D[g][M, N] = act(A[g][M, K] * B[g][N, K]^T + bias[g][N]),  g = 0..G-1
  * Both operands K-major (reduction dimension contiguous).  strideA / strideB == 0: operand shared by all g.
- * act: flag word -- bits 0-1: 1 = ELU, 2 = exact (erf) GELU (passes 2 / 4; the cgpt FFN, ref TransformerFlashAttention.py:
- * 43-57); Dpre, may be NULL, receives the pre-activation in D's layout (the GELU backward needs it, rorl_gelu_bwd_colsum); bit 2 (4, passes == 2 only) ACCUMULATE: D += result, so that a gradient with two producers (the scan's du
- * and x_proj's input gradient, ref: smamba/mamba.py:213-233) needs no separate add pass.
- * passes: 3 = 3xTF32 (fp32 parity, ~2^-21), 2 = two-term bf16 split, 3 bf16 MMAs (fp32 parity to ~2^-17 at twice
- * the tensor rate and half the operand bytes), 1 = plain TF32, 4 = the bf16 kernel's hi * hi term alone (one bf16 MMA per
- * k-step: what a layer the reference runs under bf16 autocast computes, ref TransformerFlashAttention.py:80-81).  reduce_g != 0: the G products are
- * summed into one D[M, N] (data-gradient of an ensemble layer with shared input).
- * K, N, ld*, stride* multiples of 4 (passes == 2: K a multiple of 8); bases 16-byte aligned.
- * work: device scratch of rorl_gemm_tn_work_bytes(...) bytes, 16-byte aligned (passes == 2: the kernel pre-splits
- * the B operand -- the weights, re-read by every row tile -- into bf16 hi / lo copies there); NULL otherwise.
- * transb is a flag word (passes 2 / 4 only).  Bit 1 (2): `work` ALREADY holds B's split copy -- the caller keeps it up to
- * date with rorl_split_bf16_multi after every change of the weights -- and the per-call pre-split launch is skipped (an
- * update issues ~110 GEMMs on weights that change three times).  Bit 0 (1): B is stored [K, N] with row stride ldb -- nn.Linear's weight as its input-gradient
- * GEMM needs it, EnsembleLinear's [E, in, out] weight as its forward needs it -- and the pre-split transposes it.
+ * act: flag word -- bits 0-1: 1 = ELU, 2 = exact (erf) GELU (the cgpt FFN, ref TransformerFlashAttention.py:43-57);
+ * Dpre, may be NULL, receives the pre-activation in D's layout (the GELU backward needs it, rorl_gelu_bwd_colsum);
+ * bit 2 (4) ACCUMULATE: D += result, so that a gradient with two producers (the scan's du and x_proj's input
+ * gradient, ref: smamba/mamba.py:213-233) needs no separate add pass.
+ * passes: 2 = the two-term bf16 split, 3 bf16 MMAs (fp32 parity to ~2^-17); 4 = its hi * hi term alone (one bf16 MMA
+ * per k-step: what a layer the reference runs under bf16 autocast computes, ref TransformerFlashAttention.py:80-81).
+ * Any other value: RORL_ERR_ARG.  reduce_g != 0: the G products are summed into one D[M, N] (data-gradient of an
+ * ensemble layer with shared input).
+ * K, N, ld*, stride* multiples of 4; bases 16-byte aligned.
+ * work: device scratch of rorl_gemm_tn_work_bytes(...) bytes, 16-byte aligned: the kernel pre-splits the B operand --
+ * the weights, re-read by every row tile -- into its bf16 copy there: hi [GB][N][Kp] followed by lo [GB][N][Kp], with
+ * GB = G if B is batched (strideB != 0), else 1, and Kp = K rounded up to a multiple of 8 (columns K..Kp-1 are neither
+ * written nor read).
+ * transb is a flag word.  Bit 1 (2): `work` ALREADY holds B's split copy -- the caller keeps it up to date with
+ * rorl_split_bf16_multi after every change of the weights -- and the per-call pre-split launch is skipped (an update
+ * issues ~110 GEMMs on weights that change three times).  Bit 0 (1): B is stored [K, N] with row stride ldb --
+ * nn.Linear's weight as its input-gradient GEMM needs it, EnsembleLinear's [E, in, out] weight as its forward needs
+ * it -- and the pre-split transposes it.
  * ---------------------------------------------------------------------------------------------- */
+/* bytes of `work` for rorl_gemm_tn: 2 * GB * N * Kp bf16; RORL_ERR_ARG for passes other than 2 / 4 */
 int64_t rorl_gemm_tn_work_bytes(int64_t N, int64_t K, int64_t G, int64_t strideB, int passes);
 /* (Re)build the split copies of many B operands in one launch.  jobs: DEVICE array of njobs records
  *   struct { const float* src; void* dst; int32_t N, K, G, transposed; int64_t ld, gs; }      (48 bytes each)
  * src: G groups (group stride gs floats) of [N, K] rows with row stride ld, or -- transposed != 0 -- of [K, N] rows;
- * dst: rorl_gemm_tn_work_bytes(N, K, G, gs, 2) bytes, the buffer to hand to rorl_gemm_tn as `work` with transb bit 1. */
+ * dst: rorl_gemm_tn_work_bytes(N, K, G, gs, 2) bytes, receives hi [G][N][Kp] then lo [G][N][Kp] (Kp = K rounded up
+ * to 8): the buffer to hand to rorl_gemm_tn as `work` with transb bit 1. */
 int rorl_split_bf16_multi(const void* jobs, int64_t njobs, cudaStream_t stream);
 int rorl_gemm_tn(const float* A, const float* B, const float* bias, float* D, float* Dpre, int64_t M, int64_t N, int64_t K, int64_t G,
                  int64_t lda, int64_t ldb, int64_t ldd, int64_t strideA, int64_t strideB, int64_t strideD,
@@ -246,7 +253,7 @@ int rorl_gemm_tn(const float* A, const float* B, const float* bias, float* D, fl
 /* Weight-gradient form: D[s][g][M, N] = sum over the s-th slice of rows r of A[g][r, M]^T B[g][r, N] (both operands
  * row-major with the REDUCTION over rows, i.e. MN-major for the tensor core; no transposed copies).  Split-K over
  * the R rows: splits = rorl_gemm_nt_splits(M, N, R, G); partial s lands at D + s * strideSplit and the caller sums
- * the partials (deterministic).  M, N, ld*, stride* multiples of 4. */
+ * the partials (deterministic).  M, N, ld*, stride* multiples of 4; passes 2 or 4 as for rorl_gemm_tn. */
 int rorl_gemm_nt_splits(int64_t M, int64_t N, int64_t R, int64_t G);
 int rorl_gemm_nt(const float* A, const float* B, float* D, int64_t M, int64_t N, int64_t R, int64_t G, int64_t lda,
                  int64_t ldb, int64_t ldd, int64_t strideA, int64_t strideB, int64_t strideD, int64_t splits,

@@ -81,6 +81,6 @@ int rorl_traj_gather(const float* ring, int64_t F, const int64_t* plan, int64_t 
     RORL_RETURN_LAUNCH();
 }
 
-int rorl_abi_version(void) { return 5; }   // 5: rorl_gemm_tn transb, segmented addressing in the skinny projections, rorl_skinny_dgrad
+int rorl_abi_version(void) { return 6; }   // 6: rorl_gemm_tn / rorl_gemm_nt take passes 2 and 4 only (the TF32 forms are gone); K % 4 for every form
 
 }  // extern "C"

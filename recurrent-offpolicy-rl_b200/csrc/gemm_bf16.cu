@@ -1,14 +1,15 @@
 // tcgen05 GEMM with fp32 parity from a two-term bf16 split ("bf16x3"), sm_100a.
 //
-//   D[g][M, N] = act( A[g][M, K] * B[g][N, K]^T + bias[g][N] )        (same contract as gemm.cu, passes = 2)
+//   D[g][M, N] = act( A[g][M, K] * B[g][N, K]^T + bias[g][N] )        g = 0..G-1 (ensemble members)
 //
-// Every fp32 operand element is split as x = hi + lo with hi = bf16(x), lo = bf16(x - hi) (16 mantissa bits kept; the
-// dropped lo*lo term and the representation remainder are ~2^-17 relative) and the product is accumulated as
-// lo*hi + hi*lo + hi*hi on tcgen05.mma.kind::f16 into the fp32 TMEM accumulator.  Against the 3xTF32 form of gemm.cu
-// (ref for the GEMMs it replaces: offpolicy_rnn/models/ensemble_linear_model.py:36-49, smamba/mamba.py:176,231-233,252):
-//   * the bf16 MMA runs at twice the TF32 rate (K = 16 per instruction instead of 8): 6 instead of 12 MMAs per 32-deep
-//     k-stage;
-//   * the MMA reads bf16 tiles: 72 KiB of shared-memory operand reads per stage at 128 x 256 instead of 144 KiB.
+// Replaces the cuBLAS fp32 SGEMMs behind nn.Linear / EnsembleLinear on the update path (ref:
+// offpolicy_rnn/models/ensemble_linear_model.py:36-49 einsum -> bmm; smamba in/x/dt/out_proj, ref:
+// offpolicy_rnn/models/smamba/mamba.py:176,231-233,252).  The reference runs these in true fp32 (TF32 is never enabled
+// there), so one low-precision MMA per product is not enough for the 1e-3 parity budget: every fp32 operand element is
+// split as x = hi + lo with hi = bf16(x), lo = bf16(x - hi) (16 mantissa bits kept; the dropped lo*lo term and the
+// representation remainder are ~2^-17 relative) and the product is accumulated as lo*hi + hi*lo + hi*hi on
+// tcgen05.mma.kind::f16 into the fp32 TMEM accumulator (passes = 2).  passes = 4 issues the hi*hi term alone: what a
+// layer the reference runs under bf16 autocast computes.
 // Structure (one persistent CTA per SM, 14 warps), two decoupled shared-memory rings:
 //   warp 0      TMA producer: raw fp32 A tiles (SWIZZLE_128B, 32 fp32 of K per row) into the RAW ring, and the B operand's
 //               bf16 hi / lo tiles (pre-split once per call by split_bf16_kernel: B is the small, endlessly re-read
@@ -19,7 +20,12 @@
 //               memory wavefronts -- splitter 768 + tensor core 576 + epilogue 260 per stage -- were the bound, l1tex
 //               data pipe 69 % busy with the tensor pipe at 30 %; B was two thirds of the splitter's traffic.)
 //   warp 1      MMA issuer: 2 k-steps x 3 tcgen05.mma.kind::f16 (M128 x N{128,256} x K16) per split stage
-//   warps 6-13  epilogue (identical to gemm.cu): tcgen05.ld, + bias, ELU, transposition through shared memory, 128-B rows
+//   warps 6-13  epilogue: two warps per TMEM lane quarter, each owning half of the accumulator's 32-column chunks:
+//               tcgen05.ld, + bias, ELU / GELU, shared-memory transposition, 128-B-row global stores; overlaps the next
+//               tile's main loop (double-buffered TMEM).  One warp per scheduler was latency bound (ncu: the epilogue,
+//               not the MMA, set the tile time), hence eight
+// K only has to be a multiple of 4: B's split copy pads its rows to Kp = K rounded up to 8 (16-byte rows for the
+// tensor map) while the map's extent stays K, so TMA zero-fills columns K..Kp-1 and the padding is never written or read.
 #include "common.cuh"
 #include "tc.cuh"
 #include <cuda_bf16.h>
@@ -27,18 +33,6 @@
 namespace rorl {
 
 constexpr int kBfBM = 128, kBfBK = 32;
-// Weight-gradient (NT) form, two interchangeable operand layouts for the tensor core:
-//   default            the splitters TRANSPOSE while they split (LDS.32 down the columns) into K-major SWIZZLE_64B tiles;
-//   -DRORL_NT_MNMAJOR  no transposition: MN-major SWIZZLE_128B tiles (vectorised LDS.128 / STS.128 splitters, a_major /
-//                      b_major set in the instruction descriptor).  Bit-identical results (tests/test_gemm_gpu.py passes
-//                      with either); measured 246 vs 230 us on the efc-8 dW shape and 33.4 vs 32.6 us on 256 x 256, i.e.
-//                      the splitter's transposition is not what bounds this form -- both operands being split per
-//                      128 x 128 tile is -- so the transposing form stays the default.
-#ifdef RORL_NT_MNMAJOR
-constexpr bool kNtMnMajor = true;
-#else
-constexpr bool kNtMnMajor = false;
-#endif
 constexpr int kBfThreads = 448;
 constexpr int kBfEpiWarps = 8;
 constexpr int kBfStaging = kBfEpiWarps * 32 * 128;
@@ -95,7 +89,8 @@ __device__ __forceinline__ void split8(const float4& a, const float4& b, uint4& 
 // row-major with the REDUCTION over rows (MN-major): TMA delivers each operand as 4 boxes of [32 reduction rows][32 MN
 // columns]; the splitters transpose while they split (kind::f16 multiplies K-major operands), writing K-major
 // SWIZZLE_64B bf16 rows (row = MN index, 32 reduction values = 64 B) into the split ring -- a separate buffer, so no
-// in-place hazard and no block barrier, unlike the TF32 form in gemm.cu; split-K partials as there.
+// in-place hazard and no block barrier.  Split-K over the (very long) token dimension: partial s is written at
+// D + s * strideSplit and the caller sums the partials (deterministic, no atomics).
 template <int BN, bool MN, bool ACC = false>
 __global__ void __launch_bounds__(kBfThreads, 1)
 gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapBhi,
@@ -189,7 +184,7 @@ gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
     } else if (warp == 1) {
         // ------------------------------------------------------------------ MMA issuer
         if (lane == 0) {
-            const uint32_t idesc = (MN && kNtMnMajor) ? idesc_bf16_mn(kBfBM, BN) : idesc_bf16(kBfBM, BN);
+            const uint32_t idesc = idesc_bf16(kBfBM, BN);
             uint32_t it = 0, tcount = 0;
             for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++tcount) {
                 const int acc = tcount & 1;
@@ -201,20 +196,12 @@ gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
                     mbar_wait(bar_split_full(s), (it / SS) & 1);
                     tc_fence_after();
                     const uint32_t st = split_base + s * Cfg::kSplit;
-                    uint64_t a_hi, a_lo, b_hi, b_lo;
-                    if (MN && kNtMnMajor) {        // MN-major tiles: [64-column group][32 k rows][128 B], groups 4 KiB apart
-                        a_hi = make_mnmajor_desc(st, 4096, 1024); a_lo = make_mnmajor_desc(st + Cfg::kHalfA, 4096, 1024);
-                        b_hi = make_mnmajor_desc(st + 2 * Cfg::kHalfA, 4096, 1024);
-                        b_lo = make_mnmajor_desc(st + 2 * Cfg::kHalfA + Cfg::kHalfB, 4096, 1024);
-                    } else {
-                        a_hi = make_kmajor_desc_sw64(st); a_lo = make_kmajor_desc_sw64(st + Cfg::kHalfA);
-                        b_hi = make_kmajor_desc_sw64(st + 2 * Cfg::kHalfA);
-                        b_lo = make_kmajor_desc_sw64(st + 2 * Cfg::kHalfA + Cfg::kHalfB);
-                    }
+                    const uint64_t a_hi = make_kmajor_desc_sw64(st), a_lo = make_kmajor_desc_sw64(st + Cfg::kHalfA);
+                    const uint64_t b_hi = make_kmajor_desc_sw64(st + 2 * Cfg::kHalfA);
+                    const uint64_t b_lo = make_kmajor_desc_sw64(st + 2 * Cfg::kHalfA + Cfg::kHalfB);
 #pragma unroll
                     for (int k = 0; k < kBfBK / 16; ++k) {
-                        // K-major: 32 B per k-step inside the 64-B swizzle row; MN-major: 16 k rows = two 1 KiB atoms
-                        const uint64_t adv = (MN && kNtMnMajor) ? (uint64_t)(k * 2048 >> 4) : (uint64_t)(k * 16 * 2 >> 4);
+                        const uint64_t adv = (uint64_t)(k * 16 * 2 >> 4);       // 32 B per k-step inside the 64-B swizzle row
                         const uint32_t first = (kt | k) == 0 ? 0u : 1u;
                         if (!p.single) {
                             umma_bf16(tmem_d, a_lo + adv, b_hi + adv, idesc, first);
@@ -241,33 +228,8 @@ gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
                 mbar_wait(bar_split_empty(ss), ((it / SS) & 1) ^ 1);
                 const uint8_t* raw = base_ptr + rs * Cfg::kRaw;
                 uint8_t* sp = split_ptr + ss * Cfg::kSplit;
-                if (MN && kNtMnMajor) {
-                    // No transposition: the tensor core takes MN-major operands.  item = (reduction row r, 64-column group g,
-                    // 16-byte output chunk oc = 8 columns): two raw chunks of box 2g + (oc >> 2) become chunk oc of the
-                    // 128-byte bf16 row (g, r), SWIZZLE_128B on both sides.  A quarter-warp covers one output row (8 distinct
-                    // chunks); its second half reads its odd raw chunk first so the two boxes' reads fall in different banks.
-#pragma unroll
-                    for (int op = 0; op < 2; ++op) {
-                        const uint8_t* src = raw + op * Cfg::kRawA;
-                        uint8_t* dhi = sp + (op ? 2 * Cfg::kHalfA : 0);
-                        const int half = op ? Cfg::kHalfB : Cfg::kHalfA;
-#pragma unroll
-                        for (int pass = 0; pass < 4; ++pass) {
-                            const int pr = pass * 16 + (t >> 3), oc = t & 7;
-                            const int g = pr & 1, r = pr >> 1;
-                            const int c = 2 * (oc & 3), sw = oc >> 2;
-                            const uint8_t* row = src + (2 * g + sw) * 4096 + r * 128;
-                            const float4 f0 = *reinterpret_cast<const float4*>(row + (((c + sw) ^ (r & 7)) << 4));
-                            const float4 f1 = *reinterpret_cast<const float4*>(row + (((c + 1 - sw) ^ (r & 7)) << 4));
-                            uint4 hi, lo;
-                            split8(sw ? f1 : f0, sw ? f0 : f1, hi, lo);
-                            uint8_t* dst = dhi + g * 4096 + r * 128 + ((oc ^ (r & 7)) << 4);
-                            *reinterpret_cast<uint4*>(dst) = hi;
-                            *reinterpret_cast<uint4*>(dst + half) = lo;
-                        }
-                    }
-                } else if (MN) {
-                                        // thread = (32-column box blk, MN column mn of it = lane): for each of the 4 chunks of 8 reduction rows,
+                if (MN) {
+                    // thread = (32-column box blk, MN column mn of it = lane): for each of the 4 chunks of 8 reduction rows,
                     // 8 conflict-free LDS.32 down the column (a warp reads one 128-byte raw row per instruction), split,
                     // one 16-byte store per half into row blk * 32 + lane of the K-major bf16 tile
                     const int blk = t >> 5;
@@ -314,7 +276,7 @@ gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
             }
         }
     } else {
-        // ------------------------------------------------------------------ epilogue (as in gemm.cu)
+        // ------------------------------------------------------------------ epilogue
         const int q = warp & 3;
         const int hf = (warp - 6) >> 2;
         uint8_t* stg = staging + (warp - 6) * 4096;
@@ -422,34 +384,41 @@ static int bf_sms() {
     return sms;
 }
 
-// fp32 [G][rows, cols] (row stride ld, group stride gs) -> contiguous bf16 hi / lo [G][rows, cols]
+// Row stride (bf16 elements) of B's split copy: K rounded up to 8, so that every row is a 16-byte multiple as the tensor
+// map requires.  The columns K..Kp-1 are never written: the map's extent is K and TMA zero-fills beyond it.
+__host__ __device__ constexpr long long padded_k(long long K) { return (K + 7) & ~7LL; }
+
+// fp32 [G][rows, cols] (row stride ld, group stride gs) -> bf16 hi / lo [G][rows, Kp] (Kp = padded_k(cols))
 __global__ void __launch_bounds__(256) split_bf16_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ hi,
                                                          __nv_bfloat16* __restrict__ lo, int rows, int cols, long long ld, long long gs,
                                                          long long total4) {
+    const long long Kp = padded_k(cols);
     for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < total4; i += (long long)gridDim.x * 256) {
         const long long e = i * 4;
         const int c = (int)(e % cols);
         const long long rg = e / cols;
         const int r = (int)(rg % rows);
         const long long g = rg / rows;
+        const long long o = rg * Kp + c;
         const float4 v = *reinterpret_cast<const float4*>(w + g * gs + (long long)r * ld + c);
         const __nv_bfloat162 h0 = __floats2bfloat162_rn(v.x, v.y), h1 = __floats2bfloat162_rn(v.z, v.w);
         const uint32_t u0 = *reinterpret_cast<const uint32_t*>(&h0), u1 = *reinterpret_cast<const uint32_t*>(&h1);
         const __nv_bfloat162 l0 = __floats2bfloat162_rn(v.x - __uint_as_float(u0 << 16), v.y - __uint_as_float(u0 & 0xFFFF0000u));
         const __nv_bfloat162 l1 = __floats2bfloat162_rn(v.z - __uint_as_float(u1 << 16), v.w - __uint_as_float(u1 & 0xFFFF0000u));
-        *reinterpret_cast<uint2*>(hi + e) = make_uint2(u0, u1);
-        *reinterpret_cast<uint2*>(lo + e) = make_uint2(*reinterpret_cast<const uint32_t*>(&l0), *reinterpret_cast<const uint32_t*>(&l1));
+        *reinterpret_cast<uint2*>(hi + o) = make_uint2(u0, u1);
+        *reinterpret_cast<uint2*>(lo + o) = make_uint2(*reinterpret_cast<const uint32_t*>(&l0), *reinterpret_cast<const uint32_t*>(&l1));
     }
 }
 
-// the same from the TRANSPOSED source: fp32 [G][K rows, N cols] (row stride ld) -> bf16 hi / lo [G][N, K].  nn.Linear's
+// the same from the TRANSPOSED source: fp32 [G][K rows, N cols] (row stride ld) -> bf16 hi / lo [G][N, Kp].  nn.Linear's
 // input-gradient GEMM multiplies by W, not W^T; the K-major copy the MMA wants is made here instead of by an ATen transposition.
 __global__ void __launch_bounds__(256) split_bf16_t_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ hi,
                                                            __nv_bfloat16* __restrict__ lo, int N, int K, long long ld, long long gs) {
     __shared__ float tile[32][33];
     const int n0 = blockIdx.x * 32, k0 = blockIdx.y * 32, tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+    const long long Kp = padded_k(K);
     w += (long long)blockIdx.z * gs;
-    const long long obase = (long long)blockIdx.z * N * K;
+    const long long obase = (long long)blockIdx.z * N * Kp;
     for (int j = ty; j < 32; j += 8) {
         const int k = k0 + j, n = n0 + tx;
         tile[j][tx] = (k < K && n < N) ? __ldg(w + (long long)k * ld + n) : 0.f;
@@ -460,18 +429,18 @@ __global__ void __launch_bounds__(256) split_bf16_t_kernel(const float* __restri
         if (n < N && k < K) {
             const float x = tile[tx][j];
             const __nv_bfloat16 h = __float2bfloat16_rn(x);
-            hi[obase + (long long)n * K + k] = h;
-            lo[obase + (long long)n * K + k] = __float2bfloat16_rn(x - __bfloat162float(h));
+            hi[obase + (long long)n * Kp + k] = h;
+            lo[obase + (long long)n * Kp + k] = __float2bfloat16_rn(x - __bfloat162float(h));
         }
     }
 }
 
 // Many B operands in one launch: job j = one operand (G groups of [N, K], source either [N, K] rows or, transposed, [K, N]
-// rows with row stride ld) -> its bf16 hi | lo copy in the layout gemm_tn_bf16x3 reads.  grid = (32 x 32 tiles, jobs);
+// rows with row stride ld) -> its bf16 hi | lo copy in the layout rorl_gemm_tn reads.  grid = (32 x 32 tiles, jobs);
 // the jobs table lives in device memory (it is static: weights sit in fixed arenas, the copies in persistent buffers).
 struct SplitJob {
     const float* src;
-    __nv_bfloat16* dst;          // hi at dst, lo at dst + G * N * K
+    __nv_bfloat16* dst;          // hi [G][N][Kp] at dst, lo at dst + G * N * Kp
     int N, K, G, transposed;
     long long ld, gs;
 };
@@ -480,15 +449,16 @@ __global__ void __launch_bounds__(256) split_bf16_multi_kernel(const SplitJob* _
     const SplitJob jb = jobs[blockIdx.y];
     const int tn = (jb.N + 31) / 32, tk = (jb.K + 31) / 32;
     const long long ntile = (long long)tn * tk * jb.G;
+    const long long Kp = padded_k(jb.K);
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
     __nv_bfloat16* hi = jb.dst;
-    __nv_bfloat16* lo = jb.dst + (long long)jb.G * jb.N * jb.K;
+    __nv_bfloat16* lo = jb.dst + (long long)jb.G * jb.N * Kp;
     for (long long t = blockIdx.x; t < ntile; t += gridDim.x) {
         const int g = (int)(t / ((long long)tn * tk));
         const int rem = (int)(t % ((long long)tn * tk));
         const int n0 = (rem / tk) * 32, k0 = (rem % tk) * 32;
         const float* w = jb.src + (long long)g * jb.gs;
-        const long long obase = (long long)g * jb.N * jb.K;
+        const long long obase = (long long)g * jb.N * Kp;
         __syncthreads();
         for (int j = ty; j < 32; j += 8) {
             // tile[a][b]: a = n - n0, b = k - k0
@@ -506,26 +476,21 @@ __global__ void __launch_bounds__(256) split_bf16_multi_kernel(const SplitJob* _
             if (n < jb.N && k < jb.K) {
                 const float x = tile[j][tx];
                 const __nv_bfloat16 h = __float2bfloat16_rn(x);
-                hi[obase + (long long)n * jb.K + k] = h;
-                lo[obase + (long long)n * jb.K + k] = __float2bfloat16_rn(x - __bfloat162float(h));
+                hi[obase + (long long)n * Kp + k] = h;
+                lo[obase + (long long)n * Kp + k] = __float2bfloat16_rn(x - __bfloat162float(h));
             }
         }
     }
 }
 
-int split_bf16_multi(const void* jobs, int njobs, cudaStream_t stream) {
-    if (njobs <= 0) return RORL_OK;
-    dim3 grid(64u, (unsigned)njobs);
-    split_bf16_multi_kernel<<<grid, 256, 0, stream>>>(reinterpret_cast<const SplitJob*>(jobs));
-    RORL_RETURN_LAUNCH();
-}
-
-// 3-D map over a contiguous bf16 [batch][rows][cols] tensor: box = 32 cols (64 B) x box_rows x 1, SWIZZLE_64B
-static int make_map_bf16(CUtensorMap* map, const void* ptr, long long rows, long long cols, long long batch, int box_rows) {
+// 3-D map over a bf16 [batch][rows][cols] tensor with row stride ld elements (rows contiguous, batches rows * ld apart):
+// box = 32 cols (64 B) x box_rows x 1, SWIZZLE_64B, elements beyond `cols` read as zero.
+static int make_map_bf16(CUtensorMap* map, const void* ptr, long long rows, long long cols, long long ld, long long batch,
+                         int box_rows) {
     EncodeTiledFn enc = get_encode();
     if (!enc) return RORL_ERR_ARG;
     cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, (cuuint64_t)(batch > 0 ? batch : 1)};
-    cuuint64_t strides[2] = {(cuuint64_t)cols * 2, (cuuint64_t)rows * cols * 2};
+    cuuint64_t strides[2] = {(cuuint64_t)ld * 2, (cuuint64_t)rows * ld * 2};
     cuuint32_t box[3] = {32, (cuuint32_t)box_rows, 1};
     cuuint32_t estr[3] = {1, 1, 1};
     CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(ptr), dims, strides, box, estr,
@@ -534,17 +499,33 @@ static int make_map_bf16(CUtensorMap* map, const void* ptr, long long rows, long
     return r == CUDA_SUCCESS ? RORL_OK : RORL_ERR_ARG;
 }
 
-// Called from rorl_gemm_tn_ws (gemm.cu) for passes == 2; arguments already validated there.  `bsplit`: 2 * GB * N * K
-// bf16 (GB = G if B is batched, else 1) of caller-provided scratch, filled here with B's hi | lo halves.  transb: B is
-// stored [K, N] (row stride ldb) and is transposed by the splitting pass.
-int gemm_tn_bf16x3(const float* A, const float* B, const float* bias, float* D, float* Dpre, int64_t M, int64_t N, int64_t K, int64_t G,
-                   int64_t lda, int64_t ldb, int64_t ldd, int64_t strideA, int64_t strideB, int64_t strideD,
-                   int64_t strideBias, int act, int reduce_g, int transb, int single, int force_bn, void* bsplit, cudaStream_t stream) {
-    if (!bsplit || (reinterpret_cast<uintptr_t>(bsplit) & 15)) return RORL_ERR_WORKSPACE;
-    if (K % 8) return RORL_ERR_ALIGN;                            // bf16 rows must be 16-byte multiples for the tensor map
-    const int64_t GB = strideB ? G : 1;
-    __nv_bfloat16* bhi = reinterpret_cast<__nv_bfloat16*>(bsplit);
-    __nv_bfloat16* blo = bhi + GB * N * K;
+}  // namespace rorl
+
+using namespace rorl;
+
+extern "C" {
+
+// D[g] = act(A[g] B[g]^T + bias[g]): contract in include/rorl_b200.h.  `work` receives B's bf16 hi | lo copy
+// [GB][N][Kp] (GB = G if B is batched, else 1); transb bit 0: B is stored [K, N] (row stride ldb) and is transposed by
+// the splitting pass; bit 1: `work` already holds the copy (rorl_split_bf16_multi).
+int rorl_gemm_tn(const float* A, const float* B, const float* bias, float* D, float* Dpre, int64_t M, int64_t N, int64_t K, int64_t G,
+                 int64_t lda, int64_t ldb, int64_t ldd, int64_t strideA, int64_t strideB, int64_t strideD,
+                 int64_t strideBias, int act, int passes, int reduce_g, int transb, void* work, cudaStream_t stream) {
+    if (!A || !B || !D) return RORL_ERR_ARG;
+    if (passes != 2 && passes != 4) return RORL_ERR_ARG;         // two-term split (2) or its hi * hi term alone (4)
+    if (transb & ~3) return RORL_ERR_ARG;
+    if ((act & ~7) || (act & 3) == 3) return RORL_ERR_ARG;
+    if (M <= 0 || N <= 0 || K <= 0 || G <= 0) return RORL_ERR_SHAPE;
+    if (K % 4 || N % 4 || lda % 4 || ldb % 4 || ldd % 4 || strideA % 4 || strideB % 4 || strideD % 4 || strideBias % 4)
+        return RORL_ERR_ALIGN;
+    if ((reinterpret_cast<uintptr_t>(A) | reinterpret_cast<uintptr_t>(B) | reinterpret_cast<uintptr_t>(D) |
+         reinterpret_cast<uintptr_t>(bias) | reinterpret_cast<uintptr_t>(Dpre)) & 15)
+        return RORL_ERR_ALIGN;
+    if (reduce_g && (!strideA || !strideB)) return RORL_ERR_ARG;
+    if (!work || (reinterpret_cast<uintptr_t>(work) & 15)) return RORL_ERR_WORKSPACE;
+    const int64_t GB = strideB ? G : 1, Kp = padded_k(K);
+    __nv_bfloat16* bhi = reinterpret_cast<__nv_bfloat16*>(work);
+    __nv_bfloat16* blo = bhi + GB * N * Kp;
     if (transb & 2) {
         // the caller keeps B's split copy up to date itself (rorl_split_bf16_multi after every weight change): nothing to do
     } else if (transb & 1) {
@@ -557,18 +538,19 @@ int gemm_tn_bf16x3(const float* A, const float* B, const float* bias, float* D, 
         split_bf16_kernel<<<(unsigned)nb, 256, 0, stream>>>(B, bhi, blo, (int)N, (int)K, ldb, strideB, total4);
     }
     CUtensorMap mapA, mapBhi, mapBlo;
-    const bool wide = N > 128 && force_bn != 128;
+    const bool wide = N > 128;                                   // 128 x 256 tiles read the A tile once for twice the columns
     const int bn = wide ? 256 : 128;
-    int rc = make_map(&mapA, A, M, K, lda, strideA ? G : 1, strideA, kBfBM, kBfBK);
+    int rc = make_map(&mapA, A, M, K, lda, strideA ? G : 1, strideA, kBfBM);
     if (rc) return rc;
-    rc = make_map_bf16(&mapBhi, bhi, N, K, GB, bn);
+    rc = make_map_bf16(&mapBhi, bhi, N, K, Kp, GB, bn);
     if (rc) return rc;
-    rc = make_map_bf16(&mapBlo, blo, N, K, GB, bn);
+    rc = make_map_bf16(&mapBlo, blo, N, K, Kp, GB, bn);
     if (rc) return rc;
     BfParams p;
     p.D = D; p.Dpre = Dpre; p.bias = bias; p.M = (int)M; p.N = (int)N; p.K = (int)K; p.G = (int)G;
     p.ldd = ldd; p.strideD = strideD; p.strideBias = strideBias;
-    p.a_batched = strideA != 0; p.b_batched = strideB != 0; p.act = act & 3; p.accum = (act & 4) != 0; p.reduce_g = reduce_g != 0; p.single = single != 0;
+    p.a_batched = strideA != 0; p.b_batched = strideB != 0; p.act = act & 3; p.accum = (act & 4) != 0; p.reduce_g = reduce_g != 0;
+    p.single = passes == 4;
     p.splits = 1; p.strideSplit = 0;
     const int sms = bf_sms();
     const long long tiles = ((M + kBfBM - 1) / kBfBM) * ((N + bn - 1) / bn) * (reduce_g ? 1 : G);
@@ -584,10 +566,48 @@ int gemm_tn_bf16x3(const float* A, const float* B, const float* bias, float* D, 
     RORL_RETURN_LAUNCH();
 }
 
-// Called from rorl_gemm_nt (gemm.cu) for passes == 2; arguments already validated there.
-int gemm_nt_bf16x3(const float* A, const float* B, float* D, int64_t M, int64_t N, int64_t R, int64_t G, int64_t lda, int64_t ldb,
-                   int64_t ldd, int64_t strideA, int64_t strideB, int64_t strideD, int64_t splits, int64_t strideSplit,
-                   int single, cudaStream_t stream) {
+// B operands whose split copy the CALLER maintains (transb bit 1 of rorl_gemm_tn): (re)build many of them in one launch.
+int rorl_split_bf16_multi(const void* jobs, int64_t njobs, cudaStream_t stream) {
+    if (!jobs && njobs > 0) return RORL_ERR_ARG;
+    if (njobs < 0 || njobs > 65535) return RORL_ERR_SHAPE;
+    if (njobs == 0) return RORL_OK;
+    dim3 grid(64u, (unsigned)njobs);
+    split_bf16_multi_kernel<<<grid, 256, 0, stream>>>(reinterpret_cast<const SplitJob*>(jobs));
+    RORL_RETURN_LAUNCH();
+}
+
+// bytes of `work` rorl_gemm_tn needs: B's bf16 hi | lo copies, [GB][N][Kp] each
+int64_t rorl_gemm_tn_work_bytes(int64_t N, int64_t K, int64_t G, int64_t strideB, int passes) {
+    if (passes != 2 && passes != 4) return RORL_ERR_ARG;
+    return 2 * (strideB ? G : 1) * N * padded_k(K) * 2;
+}
+
+// Split-K factor rorl_gemm_nt uses for a [M x N] output reduced over R rows in G batches (the caller sizes D with it).
+int rorl_gemm_nt_splits(int64_t M, int64_t N, int64_t R, int64_t G) {
+    if (M <= 0 || N <= 0 || R <= 0 || G <= 0) return RORL_ERR_SHAPE;
+    const long long tiles = ((M + kBfBM - 1) / kBfBM) * ((N + 127) / 128) * G;
+    const long long kt = (R + kBfBK - 1) / kBfBK;
+    long long s = (2 * 148 + tiles - 1) / tiles;
+    const long long smax = kt / 4 > 0 ? kt / 4 : 1;
+    if (s > smax) s = smax;
+    if (s < 1) s = 1;
+    return (int)s;
+}
+
+// D[s][g][M, N] = sum over the s-th slice of rows r of A[g][r, M]^T B[g][r, N]   (both operands MN-major: the
+// reduction runs over ROWS).  Weight gradients: dW[n, k] = sum_m dY[m, n] X[m, k] with A = dY, B = X.
+// splits must equal rorl_gemm_nt_splits(M, N, R, G); the caller sums the partials over s.
+int rorl_gemm_nt(const float* A, const float* B, float* D, int64_t M, int64_t N, int64_t R, int64_t G, int64_t lda,
+                 int64_t ldb, int64_t ldd, int64_t strideA, int64_t strideB, int64_t strideD, int64_t splits,
+                 int64_t strideSplit, int passes, cudaStream_t stream) {
+    if (!A || !B || !D) return RORL_ERR_ARG;
+    if (passes != 2 && passes != 4) return RORL_ERR_ARG;
+    if (M <= 0 || N <= 0 || R <= 0 || G <= 0 || splits <= 0) return RORL_ERR_SHAPE;
+    if (M % 4 || N % 4 || lda % 4 || ldb % 4 || ldd % 4 || strideA % 4 || strideB % 4 || strideD % 4 || strideSplit % 4)
+        return RORL_ERR_ALIGN;
+    if ((reinterpret_cast<uintptr_t>(A) | reinterpret_cast<uintptr_t>(B) | reinterpret_cast<uintptr_t>(D)) & 15)
+        return RORL_ERR_ALIGN;
+    if (splits != rorl_gemm_nt_splits(M, N, R, G)) return RORL_ERR_ARG;
     CUtensorMap mapA, mapB;
     int rc = make_map(&mapA, A, R, M, lda, strideA ? G : 1, strideA, kBfBK);
     if (rc) return rc;
@@ -596,7 +616,7 @@ int gemm_nt_bf16x3(const float* A, const float* B, float* D, int64_t M, int64_t 
     BfParams p;
     p.D = D; p.Dpre = nullptr; p.bias = nullptr; p.M = (int)M; p.N = (int)N; p.K = (int)R; p.G = (int)G;
     p.ldd = ldd; p.strideD = strideD; p.strideBias = 0;
-    p.a_batched = strideA != 0; p.b_batched = strideB != 0; p.act = 0; p.accum = 0; p.reduce_g = 0; p.single = single != 0;
+    p.a_batched = strideA != 0; p.b_batched = strideB != 0; p.act = 0; p.accum = 0; p.reduce_g = 0; p.single = passes == 4;
     p.splits = (int)splits; p.strideSplit = strideSplit;
     const int sms = bf_sms();
     const long long tiles = ((M + kBfBM - 1) / kBfBM) * ((N + 127) / 128) * G * splits;
@@ -605,4 +625,4 @@ int gemm_nt_bf16x3(const float* A, const float* B, float* D, int64_t M, int64_t 
     RORL_RETURN_LAUNCH();
 }
 
-}  // namespace rorl
+}  // extern "C"

@@ -5,7 +5,7 @@
 //
 // Replaces torch.nn.GRU(256, 256, batch_first=True) on the `gru` encoder path
 // (ref: offpolicy_rnn/models/rnn_base.py:59,245-247,454; cuDNN on GPU, ATen loop on CPU).
-// gi = x W_ih^T + b_ih for all steps is ONE tensor-core GEMM up front (csrc/gemm.cu); this file is
+// gi = x W_ih^T + b_ih for all steps is ONE tensor-core GEMM up front (csrc/gemm_bf16.cu); this file is
 // the L dependent steps that remain.
 //
 // Design.  W_hh is 3H x H fp32 = 786 KB at H = 256: more than one SM's shared memory, so a cluster

@@ -6,7 +6,7 @@
 //
 // Replaces torch.nn.LSTM(in, H, batch_first=True) on the `lstm` encoder path (ref: offpolicy_rnn/models/rnn_base.py,
 // layer table entry 'lstm'; cuDNN on GPU, ATen loop on CPU).  gi for all steps is ONE tensor-core GEMM up front
-// (csrc/gemm.cu); this file is the L dependent steps that remain.
+// (csrc/gemm_bf16.cu); this file is the L dependent steps that remain.
 //
 // Design.  W_hh is 4H x H fp32 = 1 MiB at H = 256, four times one SM's shared memory and four times its register
 // file.  The GRU's split (csrc/gru.cu: 64 units per CTA) would need a whole register file per CTA for weights alone,

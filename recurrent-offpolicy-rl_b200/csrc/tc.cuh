@@ -1,4 +1,4 @@
-// tcgen05 / TMEM / TMA helpers shared by the tensor-core kernels (gemm.cu, attn.cu), sm_100a only.
+// tcgen05 / TMEM / TMA helpers shared by the tensor-core kernels (gemm_bf16.cu, attn.cu), sm_100a only.
 #pragma once
 #include "common.cuh"
 #include <cuda.h>
@@ -9,12 +9,6 @@ __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* map
     asm volatile(
         "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
         ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accum) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accum) : "memory");
 }
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
@@ -32,7 +26,7 @@ __device__ __forceinline__ uint64_t make_kmajor_desc(uint32_t saddr) {
     d |= (uint64_t)2 << 61;                            // SWIZZLE_128B
     return d;
 }
-// K-major, SWIZZLE_64B (rows of 64 B = 16 fp32): 8-row groups are 512 B apart.
+// K-major, SWIZZLE_64B (rows of 64 B = 32 bf16): 8-row groups are 512 B apart.
 __device__ __forceinline__ uint64_t make_kmajor_desc_sw64(uint32_t saddr) {
     uint64_t d = 0;
     d |= (uint64_t)((saddr & 0x3FFFF) >> 4);
@@ -40,19 +34,6 @@ __device__ __forceinline__ uint64_t make_kmajor_desc_sw64(uint32_t saddr) {
     d |= (uint64_t)(512 >> 4) << 32;
     d |= (uint64_t)1 << 46;
     d |= (uint64_t)4 << 61;                            // SWIZZLE_64B
-    return d;
-}
-
-// MN-major, SWIZZLE_128B: rows of 128 B hold 64 consecutive bf16 along M (or N) for ONE k; 8 consecutive k rows form a
-// 1024-byte swizzle atom.  Canonical form (cute/atom/mma_traits_sm100.hpp, make_umma_desc<Major::MN>, in 16-byte units):
-// ((8, n), (8, k)) : ((1, LBO), (8, SBO)) -- LBO = distance between 64-element MN groups, SBO = between 8-row k groups.
-__device__ __forceinline__ uint64_t make_mnmajor_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-    uint64_t d = 0;
-    d |= (uint64_t)((saddr & 0x3FFFF) >> 4);
-    d |= (uint64_t)(lbo_bytes >> 4) << 16;
-    d |= (uint64_t)(sbo_bytes >> 4) << 32;
-    d |= (uint64_t)1 << 46;
-    d |= (uint64_t)2 << 61;                            // SWIZZLE_128B
     return d;
 }
 
@@ -66,8 +47,6 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint6
 __device__ __forceinline__ uint32_t idesc_bf16(int M, int N) {
     return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
-// the same with both operands MN-major (a_major = bit 15, b_major = bit 16)
-__device__ __forceinline__ uint32_t idesc_bf16_mn(int M, int N) { return idesc_bf16(M, N) | (1u << 15) | (1u << 16); }
 // 32 TMEM lanes (this warp's quarter) x 32 consecutive fp32 columns -> 32 registers per lane (lane = row)
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
     asm volatile(
@@ -101,15 +80,15 @@ static inline EncodeTiledFn get_encode() {
 // 3-D map over a row-major [batch][rows][cols] fp32 tensor: box = 32 cols (128 B) x box_rows x 1, SWIZZLE_128B,
 // out-of-bounds elements read as zero.
 static inline int make_map(CUtensorMap* map, const float* ptr, long long rows, long long cols, long long ld, long long batch,
-                    long long batch_stride, int box_rows, int box_cols = 32) {
+                    long long batch_stride, int box_rows) {
     EncodeTiledFn enc = get_encode();
     if (!enc) return RORL_ERR_ARG;
     cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, (cuuint64_t)(batch > 0 ? batch : 1)};
     cuuint64_t strides[2] = {(cuuint64_t)ld * 4, (cuuint64_t)(batch > 1 ? batch_stride : rows * ld) * 4};
-    cuuint32_t box[3] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows, 1};
+    cuuint32_t box[3] = {32, (cuuint32_t)box_rows, 1};
     cuuint32_t estr[3] = {1, 1, 1};
     CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(ptr), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, box_cols == 16 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                      CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     return r == CUDA_SUCCESS ? RORL_OK : RORL_ERR_ARG;
 }

@@ -614,7 +614,7 @@ class SSMCore(Function):
         x_dbl = gemm_tn(xs2, Wx)                                              # [M, R + 2N]
         Wdt_c, A_c, D_c, b_c = _f32c(Wdt), _f32c(A_log), _f32c(Dskip), _f32c(dt_bias)
         delta = torch.empty((B, L, Dn), device=xs.device, dtype=torch.float32)
-        if R % 8 == 0 and GEMM_PASSES == 2 and not _os.environ.get("RORL_DT_SKINNY"):
+        if R % 8 == 0:
             # K = R = 16: one half-empty k-tile on the tensor-core kernel, which then runs at the rate delta is written
             gemm_tn(x_dbl[:, :R], Wdt_c, out=delta.view(M, Dn))
         else:
@@ -793,12 +793,10 @@ def rms_norm_fn(x, weight, bias, residual=None, eps=1e-6, prenorm=False, residua
 
 
 # ------------------------------------------------------------------------------------------------
-# tcgen05 GEMM (3xTF32, fp32 parity) behind nn.Linear / EnsembleLinear
+# tcgen05 GEMM (two-term bf16 split, fp32 parity) behind nn.Linear / EnsembleLinear
 # ------------------------------------------------------------------------------------------------
-import os as _os
-# 3 = 3xTF32 split accumulation (~2^-21); 2 = two-term bf16 split on kind::f16 (~2^-17, half the tensor time and
-# operand bytes); 1 = plain TF32 (benchmarks only).  RORL_GEMM_PASSES overrides for A/B runs.
-GEMM_PASSES = int(_os.environ.get("RORL_GEMM_PASSES", "2"))
+# passes: 2 = two-term bf16 split on kind::f16 (~2^-17 relative); 4 = its hi * hi term alone, for the layers the
+# reference runs under bf16 autocast.
 GEMM_MIN_K = 32
 
 
@@ -907,19 +905,13 @@ class WeightSplitCache:
 _ACTIVE_SPLIT_CACHE = None
 
 
-def gemm_tn(A, B, bias=None, act: int = 0, reduce_g: bool = False, passes: int = None, want_pre: bool = False, transb: bool = False,
+def gemm_tn(A, B, bias=None, act: int = 0, reduce_g: bool = False, passes: int = 2, want_pre: bool = False, transb: bool = False,
             out: torch.Tensor = None, accumulate: bool = False):
     """D[g] = act(A[g] @ B[g]^T + bias[g]).  A [M, K] or [G, M, K]; B [N, K] or [G, N, K]; bias [N] or [G, N].
     transb: B is handed over as [K, N] / [G, K, N] (D = A @ B) and transposed by the kernel's own pre-split pass.
     out (unbatched only): a [M, N] destination with unit inner stride and any row stride (a column block of a wider
     buffer); accumulate: out += result, in the kernel's epilogue.
     Returns [M, N] (no batched operand, or reduce_g) or [G, M, N]."""
-    passes = int(passes or GEMM_PASSES)
-    if accumulate and (passes not in (2, 4) or A.shape[-1] % 8):  # only the bf16 kernel has the accumulating epilogue
-        out.add_(gemm_tn(A, B, bias, act, reduce_g, passes, False, transb))
-        return out
-    if transb and (passes not in (2, 4) or A.shape[-1] % 8):
-        B, transb = B.transpose(-1, -2).contiguous(), False
     A, B = _mat(A), _mat(B)
     G = max(A.shape[0] if A.dim() == 3 else 1, B.shape[0] if B.dim() == 3 else 1)
     M, K = A.shape[-2], A.shape[-1]
@@ -935,17 +927,17 @@ def gemm_tn(A, B, bias=None, act: int = 0, reduce_g: bool = False, passes: int =
     ldd = D.stride(-2)
     bias_c = None if bias is None else _f32c(bias.reshape(-1, Nn) if batched_out else bias.reshape(Nn))
     pre = torch.empty_like(D) if (want_pre and act) else None
-    if passes in (2, 4) and K % 8:
-        passes = 3 if passes == 2 else 1                                   # bf16 rows must be 16-byte multiples; such widths are not on the update path
     strideB = B.stride(0) if B.dim() == 3 else 0
     work, tflag = None, int(transb)
-    if _ACTIVE_SPLIT_CACHE is not None and passes in (2, 4):
+    if _ACTIVE_SPLIT_CACHE is not None:
         work = _ACTIVE_SPLIT_CACHE.lookup(B, transb, Nn, K, G, B.stride(-2), strideB)
         if work is not None:
             tflag |= 2                                   # the cache keeps this operand's split copy: no pre-split launch
     if work is None:
         wb = int(N.lib().rorl_gemm_tn_work_bytes(Nn, K, G, strideB, passes))
-        work = torch.empty(wb, dtype=torch.uint8, device=A.device) if wb else None
+        if wb < 0:
+            N.check(wb, "rorl_gemm_tn_work_bytes")                          # passes other than 2 / 4
+        work = torch.empty(wb, dtype=torch.uint8, device=A.device)
     N.call("rorl_gemm_tn", N.ptr(A), N.ptr(B), N.ptr(bias_c), N.ptr(D), N.ptr(pre), M, Nn, K, G, A.stride(-2), B.stride(-2), ldd,
            A.stride(0) if A.dim() == 3 else 0, strideB, M * Nn if batched_out else 0,
            Nn if (bias_c is not None and bias_c.dim() == 2) else 0, int(act) | (4 if accumulate else 0), passes,
@@ -953,7 +945,7 @@ def gemm_tn(A, B, bias=None, act: int = 0, reduce_g: bool = False, passes: int =
     return (D, pre) if want_pre else D
 
 
-def gemm_nt(A, B, passes: int = None):
+def gemm_nt(A, B, passes: int = 2):
     """D[g] = A[g]^T @ B[g] with the reduction over ROWS: A [R, M] or [G, R, M]; B [R, N] or [G, R, N] -> [M, N] or
     [G, M, N].  The weight-gradient GEMM: split-K partials from the tensor-core kernel, summed here."""
     A, B = _mat(A), _mat(B)
@@ -966,7 +958,7 @@ def gemm_nt(A, B, passes: int = None):
     D = torch.empty((splits, G, M, Nn), device=A.device, dtype=torch.float32)
     N.call("rorl_gemm_nt", N.ptr(A), N.ptr(B), N.ptr(D), M, Nn, R, G, A.stride(-2), B.stride(-2), Nn,
            A.stride(0) if A.dim() == 3 else 0, B.stride(0) if B.dim() == 3 else 0, M * Nn, splits, G * M * Nn,
-           int(passes or GEMM_PASSES), N.stream())
+           passes, N.stream())
     D = sum_leading(D)
     return D if batched else D[0]
 
@@ -980,7 +972,7 @@ class LinearTC(Function):
     dW on its MN-major split-K variant (gemm_nt); db is a column sum."""
 
     @staticmethod
-    def forward(ctx, x, weight, bias, elu, passes=None):
+    def forward(ctx, x, weight, bias, elu, passes=2):
         """elu: False / True, or 2 = exact GELU in the epilogue (bf16 kernel; the pre-activation is kept for its backward)."""
         K, Nn = weight.shape[1], weight.shape[0]
         xs = _mat(x.reshape(-1, K))
@@ -1020,21 +1012,20 @@ class LinearTC(Function):
         return dx, dw, db, None, None
 
 
-def linear_gelu_ok(x, weight, passes=None) -> bool:
-    """Can `gelu(linear(x))` run as one GEMM with the GELU in its epilogue?  (bf16 kernel: passes 2 / 4, K % 8 == 0.)"""
+def linear_gelu_ok(x, weight) -> bool:
+    """Can `gelu(linear(x))` run as one GEMM with the GELU in its epilogue?"""
     M = x.numel() // x.shape[-1]
-    return (x.is_cuda and x.dtype == torch.float32 and int(passes or GEMM_PASSES) in (2, 4) and weight.shape[1] % 8 == 0
-            and _gemm_ok(M, weight.shape[0], weight.shape[1]))
+    return x.is_cuda and x.dtype == torch.float32 and _gemm_ok(M, weight.shape[0], weight.shape[1])
 
 
-def linear_gelu(x, weight, bias=None, passes=None):
+def linear_gelu(x, weight, bias=None, passes=2):
     return LinearTC.apply(x, weight, bias, 2, passes)
 
 
-def linear(x, weight, bias=None, elu=False, passes=None):
+def linear(x, weight, bias=None, elu=False, passes=2):
     """nn.Linear forward (+ optional fused ELU).  Shapes the tensor-core kernel cannot take (K % 4, N % 4, K < 32)
-    go through cuBLAS; both are GPU paths.  passes=1: single TF32 pass (used where the reference itself runs the
-    layer in bf16 autocast), default 3xTF32 = fp32 parity."""
+    go through cuBLAS; both are GPU paths.  passes=4: one bf16 MMA per product (used where the reference itself runs
+    the layer in bf16 autocast), default 2 = two-term bf16 split, fp32 parity."""
     M = x.numel() // x.shape[-1]
     if x.is_cuda and _gemm_ok(M, weight.shape[0], weight.shape[1]):
         return LinearTC.apply(x, weight, bias, elu, passes)

@@ -24,7 +24,7 @@ class EnsembleLinear(nn.Module):
     def forward(self, x: torch.Tensor, fuse_elu: bool = False) -> torch.Tensor:
         W, E = self.weight, self.num_ensemble
         nd = x.dim()
-        # tensor-core path (tcgen05 3xTF32 GEMM, bias + ELU fused) for the two shapes the update uses:
+        # tensor-core path (tcgen05 bf16x3 GEMM, bias + ELU fused) for the two shapes the update uses:
         # a shared [.., in] input fanned out to E members, and a per-member [E, .., in] input
         if x.is_cuda and nd in (3, 4):
             per_member = x.shape[0] == E and (self.desire_ndim is None or self.desire_ndim == nd)

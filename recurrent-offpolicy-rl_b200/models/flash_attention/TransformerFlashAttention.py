@@ -7,9 +7,10 @@ names of flash_attn's MHA it embeds (`mha.Wqkv.{weight,bias}`, `mha.out_proj.{we
 What runs where:
   * attention: csrc/attn.cu (tcgen05, bf16 operands, fp32 accumulation) -- the reference runs flash-attn 2 in bf16
     autocast (ref :80-82);
-  * Wqkv / out_proj: tcgen05 GEMM, single TF32 pass (the reference runs them in bf16 under the same autocast; TF32
-    keeps 3 more mantissa bits, inside the 1e-2 budget of this path);
-  * FFN (fc1 -> GELU -> fc2), norms, output_fc: fp32 as in the reference (3xTF32 GEMM, fused add+norm kernels).
+  * Wqkv / out_proj: tcgen05 GEMM, one bf16 MMA per product (passes = 4): bf16 operands, fp32 accumulation, as the
+    reference computes them under the same autocast;
+  * FFN (fc1 -> GELU -> fc2), norms, output_fc: fp32 as in the reference (two-term bf16 split GEMM, fused add+norm
+    kernels).
 Differences, deliberate: tokens are NOT unpadded / re-padded (ref :104-121): every per-token operation runs on the
 padded [B*L] token axis, the attention kernel walks the sequences through a (start, length) work list, and the
 padding tokens are zeroed once at the end, which is what pad_input produces.  Attention-probability dropout
@@ -31,9 +32,8 @@ from ..linear import Linear
 from ..RNNHidden import InferenceParams  # noqa: F401  (re-exported under the reference's name)
 
 # The reference runs the MHA (Wqkv, attention, out_proj) under torch.cuda.amp.autocast(bfloat16) (ref :80-81): its linears
-# are single bf16 GEMMs.  4 = one bf16 MMA per k-step on the tcgen05 kernel (RORL_MHA_PASSES=1 selects the TF32 form).
-import os as _os
-BF16_AUTOCAST_PASSES = int(_os.environ.get("RORL_MHA_PASSES", "4"))
+# are single bf16 GEMMs.  4 = one bf16 MMA per k-step on the tcgen05 kernel.
+BF16_AUTOCAST_PASSES = 4
 
 
 def get_alibi_slopes(nheads: int):

@@ -1,4 +1,4 @@
-"""nn.Linear whose forward runs on the tcgen05 3xTF32 GEMM (kernels.linear) with an optional fused ELU
+"""nn.Linear whose forward runs on the tcgen05 bf16x3 GEMM (kernels.linear) with an optional fused ELU
 epilogue.  Same parameters / state_dict keys as torch.nn.Linear, so it is a drop-in for every `fc` layer and
 projection of the reference (ref: offpolicy_rnn/models/rnn_base.py:57,102-103)."""
 import torch.nn as nn

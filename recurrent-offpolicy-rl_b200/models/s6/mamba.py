@@ -1,7 +1,7 @@
 """s6 `mamba_*` encoder layer (the reference's secondary Mamba implementation) on the B200 kernels.
 
     RMSNorm (eps 1e-5)                      -> kernels.rms_norm_fn              (rorl_addnorm_*)
-    in_proj / x_proj / out_proj             -> tcgen05 3xTF32 GEMM              (rorl_gemm_*)
+    in_proj / x_proj / out_proj             -> tcgen05 bf16x3 GEMM              (rorl_gemm_*)
     mask * x -> causal depthwise conv -> SiLU -> kernels.causal_conv1d_silu     (rorl_conv1d_silu_*)
     selective scan with reset, carried state h0, D skip and SiLU(res) gate, final state
                                              -> kernels.selective_scan_tm       (rorl_selscan_*)

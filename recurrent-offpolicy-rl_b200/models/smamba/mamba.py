@@ -1,7 +1,7 @@
 """smamba encoder: a stack of pre-norm Mamba blocks on the B200 kernels.
 
     residual add + LayerNorm/RMSNorm   -> kernels.layer_norm_fn       (rorl_addnorm_*)
-    in_proj (two halves), x_proj, out_proj -> tcgen05 3xTF32 GEMM, token-major [B*L, .] (rorl_gemm_tn / _nt; no transposes)
+    in_proj (two halves), x_proj, out_proj -> tcgen05 bf16x3 GEMM, token-major [B*L, .] (rorl_gemm_tn / _nt; no transposes)
     mask * x -> causal depthwise conv -> SiLU -> kernels.causal_conv1d_silu (rorl_conv1d_silu_*)
     dt_proj (K = dt_rank <= 16)        -> narrow-input kernels (rorl_skinny_linear / rorl_skinny_wgrad);
                                           B_t / C_t are read in place from x_dbl

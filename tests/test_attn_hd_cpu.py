@@ -27,7 +27,7 @@ def test_attn_hd_abi_exports_and_version():
         assert hasattr(lib, name) and name in protos
         assert protos[name][1][-2] is ctypes.c_int64            # head_dim, just before the stream
         assert len(protos[name][1]) == len(protos[name[:-3]][1]) + 1
-    assert N.lib().rorl_abi_version() == 5
+    assert N.lib().rorl_abi_version() == 6
 
 
 @pytest.mark.parametrize("hd", [0, 4, 12, 136, 256])

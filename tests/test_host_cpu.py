@@ -19,8 +19,26 @@ def test_library_exports_every_declared_symbol():
     assert len(protos) >= 25
     missing = [n for n in protos if not hasattr(lib, n)]
     assert not missing, missing
-    assert N.lib().rorl_abi_version() == 5
+    assert N.lib().rorl_abi_version() == 6
     assert N.lib().rorl_selscan_dtile(32) == 64 and N.lib().rorl_selscan_dtile(7) < 0
+
+
+def test_gemm_abi_takes_bf16_passes_only():
+    """rorl_gemm_tn / rorl_gemm_nt take passes 2 and 4 only and refuse any other value before any CUDA call; the split
+    copy of B has rows padded to a multiple of 8 bf16; the tile / k-depth / debug switches are gone."""
+    import rorl_b200._native as N
+    L, d = N.lib(), 4096                              # never dereferenced
+    for passes in (1, 3):
+        assert L.rorl_gemm_tn(d, d, None, d, None, 128, 128, 64, 1, 64, 64, 128, 0, 0, 0, 0, 0, passes, 0, 0, d, None) == -3
+        assert L.rorl_gemm_nt(d, d, d, 128, 128, 256, 1, 128, 128, 128, 0, 0, 0, 1, 0, passes, None) == -3
+        assert L.rorl_gemm_tn_work_bytes(128, 64, 1, 0, passes) == -3
+    for N_ in (4, 260):
+        assert L.rorl_gemm_tn_work_bytes(N_, 36, 1, 0, 2) == 2 * N_ * 40 * 2
+        assert L.rorl_gemm_tn_work_bytes(N_, 36, 3, 4, 4) == 2 * 3 * N_ * 40 * 2
+    assert L.rorl_gemm_tn_work_bytes(256, 64, 1, 0, 2) == 2 * 256 * 64 * 2
+    lib = ctypes.CDLL(N.LIB_PATH)
+    for name in ("rorl_gemm_force_bn", "rorl_gemm_force_bk", "rorl_gemm_debug"):
+        assert not hasattr(lib, name), name
 
 
 def test_kernels_refuse_cpu_tensors():

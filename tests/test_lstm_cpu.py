@@ -83,7 +83,7 @@ def test_lstm_abi_exports_and_argument_checks():
         assert hasattr(lib, name) and name in N.declared_prototypes()
     L = N.lib()
     assert L.rorl_lstm_save_floats_per_step(256) == 5 * 256
-    assert L.rorl_abi_version() == 5
+    assert L.rorl_abi_version() == 6
     dummy = 4096                                  # never dereferenced: every call below fails its checks first
     fwd = lambda gi, w, out, B, Ln, H: L.rorl_lstm_fwd(gi, w, None, None, None, out, None, None, None, B, Ln, H, None)
     bwd = lambda dout, w, save, dg, B, Ln, H: L.rorl_lstm_bwd(dout, None, None, w, save, None, dg, None, None, B, Ln, H, None)

@@ -227,30 +227,20 @@ def bench_gemm():
         a = rn(M, k) if (g == 1 or k == 384) else rn(g, M, k)
         b = rn(n, k) if g == 1 else rn(g, n, k)
         bias = rn(n) if g == 1 else rn(g, n)
-        for passes in (3, 2, 1):
+        for passes in (2, 4):
             t = timeit(lambda: K.gemm_tn(a, b, bias, 1, passes=passes))
             fl = 2.0 * M * n * k * g
-            rec(f"gemm_tn {tag} passes={passes}", t, flops=fl * (3 if passes > 1 else 1), nbytes=4 * (a.numel() + b.numel() + M * n * g),
+            rec(f"gemm_tn {tag} passes={passes}", t, flops=fl * (3 if passes == 2 else 1), nbytes=4 * (a.numel() + b.numel() + M * n * g),
                 note=f"useful fp32 TFLOP/s {fl / t / 1e12:.1f}")
-        for bk in (16,):                 # A/B: 16-wide k-stages (twice as deep a ring)
-            N.lib().rorl_gemm_force_bk(bk)
-            t = timeit(lambda: K.gemm_tn(a, b, bias, 1, passes=3))
-            N.lib().rorl_gemm_force_bk(0)
-            rec(f"gemm_tn {tag} passes=3 BK={bk} (A/B)", t, flops=fl * 3, note=f"useful fp32 TFLOP/s {fl / t / 1e12:.1f}")
-        if n > 128:                      # A/B: the 128 x 128 tile on the same shape
-            N.lib().rorl_gemm_force_bn(128)
-            t = timeit(lambda: K.gemm_tn(a, b, bias, 1, passes=3))
-            N.lib().rorl_gemm_force_bn(0)
-            rec(f"gemm_tn {tag} passes=3 BN=128 (A/B)", t, flops=fl * 3, note=f"useful fp32 TFLOP/s {fl / t / 1e12:.1f}")
     # weight gradient
     gq, xq = rn(M, 256), rn(M, 256)
-    for passes in (3, 2):
+    for passes in (2, 4):
         t = timeit(lambda: K.gemm_nt(gq, xq, passes=passes))
-        rec(f"gemm_nt 256x256 R=32608 passes={passes}", t, flops=3 * 2.0 * M * 256 * 256, nbytes=4 * (gq.numel() + xq.numel()))
+        rec(f"gemm_nt 256x256 R=32608 passes={passes}", t, flops=(3 if passes == 2 else 1) * 2.0 * M * 256 * 256, nbytes=4 * (gq.numel() + xq.numel()))
     g8, x8 = rn(8, M, 256), rn(8, M, 256)
-    for passes in (3, 2):
+    for passes in (2, 4):
         t = timeit(lambda: K.gemm_nt(x8, g8, passes=passes))
-        rec(f"gemm_nt efc-8 L2 dW 8x[256x256] R=32608 passes={passes}", t, flops=3 * 2.0 * M * 256 * 256 * 8, nbytes=4 * (g8.numel() + x8.numel()))
+        rec(f"gemm_nt efc-8 L2 dW 8x[256x256] R=32608 passes={passes}", t, flops=(3 if passes == 2 else 1) * 2.0 * M * 256 * 256 * 8, nbytes=4 * (g8.numel() + x8.numel()))
     c = torch.empty(M, 256, device=dev)
     a2, w2 = rn(M, 256), rn(256, 256)
     t = timeit(lambda: torch.mm(a2, w2, out=c))

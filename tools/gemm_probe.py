@@ -13,7 +13,7 @@ dev = torch.device("cuda:0")
 M = 32 * 1019
 shapes = {"efc2": (256, 256, 8), "efc1": (256, 384, 8), "fc": (256, 256, 1), "inproj": (512, 256, 1)}
 which = (sys.argv[1] if len(sys.argv) > 1 else "efc2,fc").split(",")
-passes = [int(x) for x in (sys.argv[2] if len(sys.argv) > 2 else "3,2,1").split(",")]
+passes = [int(x) for x in (sys.argv[2] if len(sys.argv) > 2 else "2,4").split(",")]
 for name in which:
     n, k, g = shapes[name]
     a = torch.randn(M, k, device=dev) if (g == 1 or name == "efc1") else torch.randn(g, M, k, device=dev)
