@@ -191,6 +191,21 @@ int rorl_q_loss_fwd_bwd(const float* q, const float* y, const float* mask, const
 int rorl_actor_loss_fwd_bwd(const float* q, const float* logp, const float* mask, const float* nvalid,
                             const float* log_alpha, float target_entropy, int mode, float* out, float* dq,
                             float* dlogp, float* work, int64_t E, int64_t M, cudaStream_t stream);
+/* Discrete actions (ref: sac_full_length_rnn_ensembleQ.py:134-185, sac_full_length_rnn_redq.py:52-88): q [E, M, A] holds one
+ * Q per action, logp [M, A] the policy's log-probabilities; 1 <= A <= 256.
+ * rorl_discrete_target_expect: m[i] = sum_a exp(logp[i, a]) (min over the selected members of q[e, i, a] - alpha logp[i, a]),
+ * alpha = exp(log_alpha[0]); like rorl_target_minq it initialises guard min/max from m on the first call, and m feeds
+ * rorl_target_finish unchanged.
+ * rorl_discrete_actor_loss_fwd_bwd: agg = min over members (mode 0) or mean (mode 1), p = exp(logp);
+ *   out[0] = sum_i mask_i sum_a p (alpha logp - agg) / nvalid (actor loss), out[1] = sum_i mask_i sum_a p logp / nvalid;
+ *   dlogp[i, a] = mask_i / nvalid * p (alpha logp - agg + alpha).  q receives no gradient (the discrete value ignores its
+ *   action argument and its weights are frozen under the actor). */
+int rorl_discrete_target_expect(const float* q, const int32_t* sel, int64_t nsel, int64_t E, int64_t M, int64_t A,
+                                const float* logp, const float* log_alpha, float* m, double* guard, float* work,
+                                cudaStream_t stream);
+int rorl_discrete_actor_loss_fwd_bwd(const float* q, const float* logp, const float* mask, const float* nvalid,
+                                     const float* log_alpha, int mode, float* out, float* dlogp, float* work, int64_t E,
+                                     int64_t M, int64_t A, cudaStream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Multi-tensor AdamW step (+ optional Polyak target update) over a flat parameter arena.
@@ -289,6 +304,23 @@ int rorl_tanh_gaussian_fwd(const float* out, const float* noise, float* action_m
 int rorl_tanh_gaussian_bwd(const float* out, const float* noise, const float* d_mean, const float* d_sample, const float* d_log_prob,
                            float* d_out, int64_t M, int64_t A, int64_t ld_out, float min_logstd, float max_logstd,
                            cudaStream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Categorical policy head (csrc/categorical.cu), forward and backward in one kernel each.  Replaces the elementwise graph
+ * of ContextualSACDiscretePolicy.process_model_out (ref: offpolicy_rnn/policy_value_models/contextual_sac_discrete_policy.py:
+ * 106-111).  logits [M, A] with row stride ld (>= A); 1 <= A <= 256; M == 0 is a no-op.
+ *   s = softmax(logits); probs = (s + 0.01) / sum(s + 0.01); logp = log(probs)          [M, A] contiguous
+ *   mode[i] = argmax_a probs (first index on ties), written as float                    [M]
+ *   sample[i] = first a with cumsum(probs)[a] > u[i] * sum(probs), as float             [M]; u [M] uniform draws, or NULL
+ *               (no sample drawn; sample may then be NULL too)
+ * bwd: d_logits [M, A] contiguous = s * (v - sum_a s v), v = d_logp / probs / sum(s + 0.01): autograd through the ops above
+ * in closed form (the renormalising sum's gradient is uniform over a and the softmax Jacobian removes it).  Recomputes
+ * everything from the logits.
+ * ---------------------------------------------------------------------------------------------- */
+int rorl_categorical_fwd(const float* logits, int64_t ld, const float* u, float* probs, float* logp, float* mode,
+                         float* sample, int64_t M, int64_t A, cudaStream_t stream);
+int rorl_categorical_bwd(const float* logits, int64_t ld, const float* d_logp, float* d_logits, int64_t M, int64_t A,
+                         cudaStream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
  * GRU recurrence as a persistent thread-block-cluster kernel (W_hh resident in registers across a

@@ -30,6 +30,7 @@ import numpy as np
 import torch
 
 from .. import _native as N
+from .. import kernels as K
 from ..buffers.transition_buffer.nested_replay_memory import NestedMemoryArray
 from ..policy_value_models.make_models import make_policy_model, make_value_model
 from ..utility.q_value_guard import QValueGuard
@@ -280,7 +281,7 @@ class FullLengthRNNUpdate:
             m.need_full_hidden = False                  # the update never reads forward()'s per-layer output record
         gpt = any(str(t).startswith(('cgpt', 'gpt', 'transformer')) for m in (self.policy, self.values[0])
                   for t in m.embedding_network.layer_type)
-        side_ok = (self.device.type == 'cuda' and not self.discrete_env and not gpt       # cgpt: device-side dropout counter order
+        side_ok = (self.device.type == 'cuda' and not gpt       # cgpt: device-side dropout counter order
                    and os.environ.get('RORL_SIDE_STREAM', '1') != '0')
         self._side_stream = torch.cuda.Stream(device=self.device) if side_ok else None
         self._has_gru = any(str(t) == 'gru' for m in (self.policy, self.values[0]) for t in m.embedding_network.layer_type)
@@ -297,7 +298,6 @@ class FullLengthRNNUpdate:
         # by one launch per arena whenever that arena changes (kernels.WeightSplitCache)
         self._split_cache = None
         if self.device.type == 'cuda' and os.environ.get('RORL_SPLIT_CACHE', '1') != '0':
-            import rorl_b200.kernels as K
             self._split_cache = K.WeightSplitCache(self.device)
             self._split_owner = {name: self._split_cache.add_owner(a.flat) for name, a in
                                  (('policy', self.policy_arena), ('value', self.value_arena), ('target', self.target_arena))}
@@ -410,14 +410,20 @@ class FullLengthRNNUpdate:
         E, M = q_next.shape[0], q_next[0].numel()
         m = torch.empty(M, dtype=torch.float32, device=self.device)
         sel = sel_idx                                                  # int32 device tensor [m]
-        # every operand is bound to a local until both launches are enqueued: a temporary freed right after
+        # every operand is bound to a local until its launch is enqueued: a temporary freed right after
         # data_ptr() would hand its block to the next temporary and the pointers would alias.
         qn = q_next.contiguous()
         lp = None if logp_next is None else logp_next.contiguous()
-        r_c, d_c, t_c, m_c = reward.contiguous(), done.contiguous(), timeout.contiguous(), mask.contiguous()
-        y = torch.empty_like(r_c)
         N.call("rorl_target_minq", N.ptr(qn), N.ptr(sel), int(sel.numel()), E, M, N.ptr(lp), N.ptr(self.log_sac_alpha.data),
                N.ptr(m), N.ptr(self.Q_guard.state), N.ptr(self._work), N.stream())
+        return self._target_finish(m, reward, done, timeout, mask)
+
+    def _target_finish(self, m, reward, done, timeout, mask):
+        """y = r + (1 - done') * gamma * clamp(m) and the guard update, from the per-step value m [M] whose kernel has
+        initialised the guard on its first call; fills stats[0] = max|y|, stats[1] = n_valid."""
+        M = m.numel()
+        r_c, d_c, t_c, m_c = reward.contiguous(), done.contiguous(), timeout.contiguous(), mask.contiguous()
+        y = torch.empty_like(r_c)
         if self.dist_group is not None and not self._guard_init_synced:
             # very first call (always launched eagerly): the guard bounds were just initialised from THIS rank's rows;
             # make them the global extrema before the clamp / update uses them (ref: q_value_guard.py:22-27)
@@ -618,10 +624,12 @@ class FullLengthRNNUpdate:
 
     def _graph_allowed(self) -> bool:
         """CUDA-graph replay needs a launch sequence that depends on nothing the host decides per step: an injected
-        `noise_fn` (parity tests) returns a different tensor per call.  (The cgpt encoder's attention work list depends
+        `noise_fn` / `sample_fn` (parity tests) returns a different tensor per call.  (The cgpt encoder's attention work list depends
         on the length table only, which is part of the graph key; it is cached on the device by the first, eager, call.)"""
-        if not self.use_cuda_graph or self.discrete_env:
+        if not self.use_cuda_graph:
             return False
+        if self.discrete_env:      # the categorical head's default draw (sample_fn None) is an in-kernel torch.rand draw
+            return all(m.sample_fn is None or getattr(m.sample_fn, 'graph_safe', False) for m in (self.policy, self.target_policy))
         ok = lambda fn: fn is torch.randn_like or getattr(fn, 'graph_safe', False)   # device-only, same launches every call
         return all(ok(getattr(m, 'noise_fn', torch.randn_like)) for m in (self.policy, self.target_policy))
 
@@ -712,19 +720,20 @@ class FullLengthRNNUpdate:
     def _stage_target_discrete(self, c, target_policy_hidden, target_hidden):
         """Discrete actions: y = r + (1 - done) gamma clamp(sum_a pi(a|s') (min_sel Q'(s', a) - alpha log pi(a|s')))
         (ref: sac_full_length_rnn_ensembleQ.py:134-151; REDQ subset + one-hot last action: sac_full_length_rnn_redq.py:52-72).
-        The expectation over actions is formed with torch ops on [B, L, A] tensors; clamp / guard / statistics run on the
-        same fused kernels as the continuous path (the per-step scalar enters as a one-member `q`)."""
+        The expectation over actions is one kernel (rorl_discrete_target_expect, which also initialises the guard); clamp /
+        guard / statistics run on the same fused kernel as the continuous path."""
         batch, sel = c['batch'], c['sel']
         with torch.no_grad():
-            onehot = self.policy.action2onehot(batch.action.long())
+            onehot = self.policy.action2onehot(batch.action)
             lst_a = onehot if self.use_redq else batch.action                       # ref :141 (base class passes the raw index)
+            # the target critic's context encoder does not depend on the action: it runs beside the policy
+            tv_embedded = self._beside(lambda: self.target_values[0].embed(batch.next_state, batch.state, onehot, target_hidden,
+                                                                           batch.reward))
             _, _, a_next, logp_next, _, _ = self.policy.forward(batch.next_state, batch.state, lst_a, target_policy_hidden, batch.reward)
-            q_next = self.target_values[0].forward(batch.next_state, batch.state, onehot, a_next, target_hidden, batch.reward)[0]
-            q_min = q_next.index_select(0, sel.long()).min(dim=0).values              # [B, L, A]
-            alpha = self.log_sac_alpha.data.exp()
-            m = ((q_min - alpha * logp_next) * logp_next.exp()).sum(dim=-1, keepdim=True)
-            one = torch.zeros(1, dtype=torch.int32, device=self.device)
-            c['target_Q'] = self._target_Q(m.reshape(1, *m.shape), one, None, batch.reward, batch.done, batch.timeout, batch.mask)
+            q_next = self.target_values[0].forward(batch.next_state, batch.state, onehot, a_next, target_hidden, batch.reward,
+                                                   embedded=tv_embedded())[0]
+            m = K.discrete_target_expect(q_next, sel, logp_next, self.log_sac_alpha.data, self.Q_guard.state, self._work)
+            c['target_Q'] = self._target_finish(m, batch.reward, batch.done, batch.timeout, batch.mask)
         self.last_target_Q = c['target_Q']
 
     def _stage_critic(self, c, overlap):
@@ -813,34 +822,33 @@ class FullLengthRNNUpdate:
     def _actor_discrete(self, c, overlap):
         """Discrete actor: L = sum_mask sum_a pi(a|s) (alpha log pi(a|s) - agg_e Q_e(s, a)) / n_valid, agg = min (ensembleQ)
         or mean (REDQ) (ref: sac_full_length_rnn_ensembleQ.py:165-179, sac_full_length_rnn_redq.py:74-88); alpha is fixed
-        for discrete action spaces (ref: sac.py:72-74).  torch autograd over [B, L, A] tensors."""
-        batch = c['batch']
+        for discrete action spaces (ref: sac.py:72-74).  One kernel forms the loss, stats[4:6] and d loss / d logp; the
+        backward runs from logp through the categorical head (q gets no gradient: its weights are frozen and its embedding
+        detached here)."""
+        batch, mask_c = c['batch'], c['mask_c']
         n_valid = self._stats[1:2]
+        state, last_state, last_action, reward_input = batch.state, batch.last_state, batch.last_action, batch.reward_input
         for w in self.value_arena.params:
             w.requires_grad_(False)
         try:
-            _, _, a_samp, logp, _, _ = self.policy.forward(batch.state, batch.last_state, batch.last_action, c['policy_hidden'], batch.reward_input)
-            qp = self.values[0].forward(batch.state, batch.last_state, batch.last_action, a_samp, c['value_hidden'], batch.reward_input,
-                                        detach_embedding=True)[0]
+            # the critic's encoder under the actor is detached and its weights are frozen here: no graph, runs beside the policy
+            v_embedded = self._beside(lambda: self.values[0].embed(state, last_state, last_action, c['value_hidden'], reward_input))
+            _, _, a_samp, logp, _, _ = self.policy.forward(state, last_state, last_action, c['policy_hidden'], reward_input)
+            qp = self.values[0].forward(state, last_state, last_action, a_samp, c['value_hidden'], reward_input,
+                                        detach_embedding=True, embedded=v_embedded())[0]
         finally:
             for w in self.value_arena.params:
                 w.requires_grad_(True)
-        agg = qp.mean(dim=0) if self.use_redq else qp.min(dim=0).values
-        alpha = self.log_sac_alpha.data.exp()
-        probs = logp.exp()
-        per_step = ((alpha * logp - agg) * probs).sum(dim=-1, keepdim=True)
-        actor_loss = (per_step * batch.mask).sum() / n_valid
+        dlogp = K.discrete_actor_loss(qp, logp, mask_c, n_valid, self.log_sac_alpha.data, 1 if self.use_redq else 0,
+                                      self._stats[4:6], self._work)
         self.optimizer_policy.zero_grad(detach=not overlap)
         if overlap:
             self._sync_policy.begin()
-        actor_loss.backward()
+        torch.autograd.backward(logp, dlogp)
         if overlap:
             self._sync_policy.finish()
         else:
             self.policy_arena.collect()
-        with torch.no_grad():
-            self._stats[4:5].copy_(actor_loss.detach().reshape(1))
-            self._stats[5:6].copy_((((logp * probs).sum(dim=-1, keepdim=True) * batch.mask).sum() / n_valid).reshape(1))
 
     def _stage_policy_step(self, c):
         if not c['did_policy']:

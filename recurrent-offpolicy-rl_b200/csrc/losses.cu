@@ -197,6 +197,85 @@ __global__ void __launch_bounds__(kLossThreads) actor_loss_kernel(
     }
 }
 
+// Discrete actions ([E, M, A] Q, [M, A] log-probabilities): one warp per row i, lanes over the actions, so that each
+// row's expectation over actions is one fixed-order warp sum.  Rows are strided over the warps of the grid.
+constexpr int kLossWarps = kLossThreads / 32;
+
+__global__ void __launch_bounds__(kLossThreads) discrete_target_expect_kernel(
+    const float* __restrict__ q, const int32_t* __restrict__ sel, int nsel, int64_t M, int A,
+    const float* __restrict__ logp, const float* __restrict__ log_alpha, float* __restrict__ m, double* guard, float* work) {
+    __shared__ float sbuf[64];
+    const int lane = threadIdx.x & 31;
+    const float alpha = expf(log_alpha[0]);
+    float v[2] = {FLT_MAX, -FLT_MAX};
+    for (int64_t i = (int64_t)blockIdx.x * kLossWarps + (threadIdx.x >> 5); i < M; i += (int64_t)gridDim.x * kLossWarps) {
+        float acc = 0.f;
+        for (int a = lane; a < A; a += 32) {
+            float mn = FLT_MAX;
+            for (int s = 0; s < nsel; ++s) mn = fminf(mn, q[((int64_t)sel[s] * M + i) * A + a]);
+            const float lp = logp[i * A + a];
+            acc = fmaf(mn - alpha * lp, expf(lp), acc);
+        }
+        acc = warp_sum(acc);
+        if (lane == 0) {   // lanes hold the sum in different association orders: lane 0's is the one written
+            m[i] = acc;
+            v[0] = fminf(v[0], acc);
+            v[1] = fmaxf(v[1], acc);
+        }
+    }
+    const int op[2] = {1, 2};
+    if (grid_reduce<2>(v, op, work, sbuf)) {
+        if (guard[2] == 0.0) {   // first clamp() call initialises the bounds from the tensor itself
+            guard[0] = (double)v[0];
+            guard[1] = (double)v[1];
+            guard[2] = 1.0;
+        }
+    }
+}
+
+__global__ void __launch_bounds__(kLossThreads) discrete_actor_loss_kernel(
+    const float* __restrict__ q, const float* __restrict__ logp, const float* __restrict__ mask,
+    const float* __restrict__ nvalid, const float* __restrict__ log_alpha, int mode, float* __restrict__ out,
+    float* __restrict__ dlogp, float* work, int E, int64_t M, int A) {
+    __shared__ float sbuf[64];
+    const int lane = threadIdx.x & 31;
+    const float inv = 1.0f / nvalid[0];
+    const float alpha = expf(log_alpha[0]);
+    float v[2] = {0.f, 0.f};   // sum_i mask_i sum_a p (alpha logp - agg), sum_i mask_i sum_a p logp
+    for (int64_t i = (int64_t)blockIdx.x * kLossWarps + (threadIdx.x >> 5); i < M; i += (int64_t)gridDim.x * kLossWarps) {
+        const float mk = mask[i];
+        const float g = mk * inv;
+        float r = 0.f, h = 0.f;
+        for (int a = lane; a < A; a += 32) {
+            float agg;
+            if (mode == 0) {
+                agg = q[i * A + a];
+                for (int e = 1; e < E; ++e) agg = fminf(agg, q[((int64_t)e * M + i) * A + a]);
+            } else {
+                float s = 0.f;
+                for (int e = 0; e < E; ++e) s += q[((int64_t)e * M + i) * A + a];
+                agg = s / (float)E;
+            }
+            const float lp = logp[i * A + a], p = expf(lp);
+            const float t = alpha * lp - agg;
+            r = fmaf(p, t, r);
+            h = fmaf(p, lp, h);
+            dlogp[i * A + a] = g * p * (t + alpha);
+        }
+        r = warp_sum(r);
+        h = warp_sum(h);
+        if (lane == 0) {
+            v[0] = fmaf(mk, r, v[0]);
+            v[1] = fmaf(mk, h, v[1]);
+        }
+    }
+    const int op[2] = {0, 0};
+    if (grid_reduce<2>(v, op, work, sbuf)) {
+        out[0] = v[0] * inv;
+        out[1] = v[1] * inv;
+    }
+}
+
 __global__ void __launch_bounds__(kLossThreads) sumsq_kernel(const float* __restrict__ p, int64_t n, float* out,
                                                               float* work) {
     __shared__ float sbuf[64];
@@ -213,6 +292,8 @@ static int loss_grid(int64_t M) {
     if (nb < 1) nb = 1;
     return (int)nb;
 }
+
+static int loss_grid_rows(int64_t M) { return loss_grid((M + kLossWarps - 1) / kLossWarps * kLossThreads); }
 
 }  // namespace rorl
 
@@ -257,6 +338,26 @@ int rorl_actor_loss_fwd_bwd(const float* q, const float* logp, const float* mask
     if (E <= 0 || M <= 0 || (mode != 0 && mode != 1)) return RORL_ERR_SHAPE;
     actor_loss_kernel<<<loss_grid(M), kLossThreads, 0, stream>>>(q, logp, mask, nvalid, log_alpha, target_entropy, mode,
                                                                 out, dq, dlogp, work, (int)E, M);
+    RORL_RETURN_LAUNCH();
+}
+
+int rorl_discrete_target_expect(const float* q, const int32_t* sel, int64_t nsel, int64_t E, int64_t M, int64_t A,
+                                const float* logp, const float* log_alpha, float* m, double* guard, float* work,
+                                cudaStream_t stream) {
+    if (!q || !sel || !logp || !log_alpha || !m || !guard || !work) return RORL_ERR_ARG;
+    if (nsel <= 0 || nsel > E || M <= 0 || A < 1 || A > 256) return RORL_ERR_SHAPE;
+    discrete_target_expect_kernel<<<loss_grid_rows(M), kLossThreads, 0, stream>>>(q, sel, (int)nsel, M, (int)A, logp,
+                                                                                  log_alpha, m, guard, work);
+    RORL_RETURN_LAUNCH();
+}
+
+int rorl_discrete_actor_loss_fwd_bwd(const float* q, const float* logp, const float* mask, const float* nvalid,
+                                     const float* log_alpha, int mode, float* out, float* dlogp, float* work, int64_t E,
+                                     int64_t M, int64_t A, cudaStream_t stream) {
+    if (!q || !logp || !mask || !nvalid || !log_alpha || !out || !dlogp || !work) return RORL_ERR_ARG;
+    if (E <= 0 || M <= 0 || A < 1 || A > 256 || (mode != 0 && mode != 1)) return RORL_ERR_SHAPE;
+    discrete_actor_loss_kernel<<<loss_grid_rows(M), kLossThreads, 0, stream>>>(q, logp, mask, nvalid, log_alpha, mode, out,
+                                                                               dlogp, work, (int)E, M, (int)A);
     RORL_RETURN_LAUNCH();
 }
 

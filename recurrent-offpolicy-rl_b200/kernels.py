@@ -9,6 +9,8 @@ Each Function is the B200 counterpart of one autograd Function / fused op of the
   GRUScan                               <- torch.nn.GRU recurrence (ref: offpolicy_rnn/models/rnn_base.py:59,245-247,454)
   LSTMScan                              <- torch.nn.LSTM recurrence (ref: offpolicy_rnn/models/rnn_base.py layer table 'lstm')
   CausalConv1dSiLU                      <- mask * x -> nn.Conv1d -> SiLU (ref: offpolicy_rnn/models/smamba/mamba.py:207-212)
+  CategoricalHead                       <- softmax / floor / log / argmax / Categorical sample of the discrete policy
+                                           (ref: offpolicy_rnn/policy_value_models/contextual_sac_discrete_policy.py:106-111)
 
 All of them require CUDA tensors: there is no CPU implementation (the oracle under oracle/ is test
 infrastructure and is never imported from here).
@@ -283,6 +285,81 @@ class TanhGaussianHead(Function):
 
 def tanh_gaussian_head(out, noise, lo, hi):
     return TanhGaussianHead.apply(out, noise, lo, hi)
+
+
+# ------------------------------------------------------------------------------------------------
+# categorical policy head and the discrete-action losses
+# ------------------------------------------------------------------------------------------------
+class CategoricalHead(Function):
+    """(mode, sample, logp, probs) of the discrete policy from its head output [.., A] (read in place with its row stride)
+    and uniform draws u [..] (or None: no sample): one kernel forward, one backward (csrc/categorical.cu).  mode and sample
+    are float action indices [.., 1] and carry no gradient; sample is None without u.  A gradient reaching probs is
+    folded into that of logp (probs = exp(logp), so d logp += d probs * probs)."""
+
+    @staticmethod
+    def forward(ctx, logits, u):
+        A = logits.shape[-1]
+        z = logits.reshape(-1, A)
+        if z.dtype != torch.float32 or z.stride(-1) != 1:
+            z = z.float().contiguous()
+        M = z.shape[0]
+        dev = logits.device
+        probs = torch.empty((M, A), device=dev, dtype=torch.float32)
+        logp = torch.empty_like(probs)
+        mode = torch.empty((M,), device=dev, dtype=torch.float32)
+        uc = None if u is None else _f32c(u.reshape(M))
+        sample = None if u is None else torch.empty_like(mode)
+        N.call("rorl_categorical_fwd", N.ptr(z), z.stride(0) if M > 1 else A, N.ptr(uc), N.ptr(probs), N.ptr(logp), N.ptr(mode),
+               N.ptr(sample), M, A, N.stream())
+        ctx.save_for_backward(z, probs)
+        ctx.lshape = logits.shape
+        ctx.mark_non_differentiable(*([mode] if sample is None else [mode, sample]))
+        lead = logits.shape[:-1]
+        return (mode.view(*lead, 1), None if sample is None else sample.view(*lead, 1), logp.view(*lead, A),
+                probs.view(*lead, A))
+
+    @staticmethod
+    def backward(ctx, d_mode, d_sample, d_logp, d_probs):
+        z, probs = ctx.saved_tensors
+        M, A = probs.shape
+        g = None if d_logp is None else d_logp.reshape(M, A)
+        if d_probs is not None:
+            gp = d_probs.reshape(M, A) * probs
+            g = gp if g is None else g + gp
+        if g is None:
+            return None, None
+        g = _f32c(g)
+        dz = torch.empty((M, A), device=z.device, dtype=torch.float32)
+        N.call("rorl_categorical_bwd", N.ptr(z), z.stride(0) if M > 1 else A, N.ptr(g), N.ptr(dz), M, A, N.stream())
+        return dz.view(ctx.lshape), None
+
+
+def categorical_head(logits, u=None):
+    return CategoricalHead.apply(logits, u)
+
+
+def discrete_target_expect(q, sel, logp, log_alpha, guard, work):
+    """m [M] = sum_a exp(logp) (min_{e in sel} q[e] - alpha logp) for q [E, .., A], logp [.., A]; initialises the Q guard
+    on its first call (csrc/losses.cu).  sel: int32 device tensor of member indices."""
+    E, A = q.shape[0], q.shape[-1]
+    qc, lp = _f32c(q), _f32c(logp)
+    M = lp.numel() // A
+    m = torch.empty(M, device=q.device, dtype=torch.float32)
+    N.call("rorl_discrete_target_expect", N.ptr(qc), N.ptr(sel), int(sel.numel()), E, M, A, N.ptr(lp), N.ptr(log_alpha),
+           N.ptr(m), N.ptr(guard), N.ptr(work), N.stream())
+    return m
+
+
+def discrete_actor_loss(q, logp, mask, nvalid, log_alpha, mode, out, work):
+    """Discrete actor loss over q [E, .., A] (agg: mode 0 min, 1 mean) and logp [.., A] with the valid-step mask [..]:
+    writes out[0] = actor loss, out[1] = masked mean of sum_a p logp, and returns d loss / d logp (shaped like logp)."""
+    E, A = q.shape[0], q.shape[-1]
+    qc, lp, mk = _f32c(q), _f32c(logp), _f32c(mask)
+    M = lp.numel() // A
+    dlogp = torch.empty_like(lp)
+    N.call("rorl_discrete_actor_loss_fwd_bwd", N.ptr(qc), N.ptr(lp), N.ptr(mk), N.ptr(nvalid), N.ptr(log_alpha), int(mode),
+           N.ptr(out), N.ptr(dlogp), N.ptr(work), E, M, A, N.stream())
+    return dlogp
 
 
 # ------------------------------------------------------------------------------------------------

@@ -51,10 +51,18 @@ class ContextualSACDiscreteValue(ContextualModel, _InputEncoders):
             return self.uni_model_input_mapping_activation_func(self.state_input_encoder(state))
         return self.state_input_encoder(state)
 
-    def forward(self, state, lst_state, lst_action, action, rnn_memory: Optional[RNNHidden], reward, detach_embedding=False):
-        emb_in = self.get_embedding_input(state, lst_state, lst_action, reward)
-        value, rnn_memory, emb, full = self.meta_forward(emb_in, self.state_encoding(state), rnn_memory, detach_embedding)
+    def forward(self, state, lst_state, lst_action, action, rnn_memory: Optional[RNNHidden], reward, detach_embedding=False,
+                embedded=None):
+        """embedded: what `embed(...)` returned for the same (state, lst_state, lst_action, rnn_memory, reward), so that a
+        caller may run the context encoder ahead of (or beside) the policy, as for the continuous value."""
+        emb_in = None if embedded is not None else self.get_embedding_input(state, lst_state, lst_action, reward)
+        value, rnn_memory, emb, full = self.meta_forward(emb_in, self.state_encoding(state), rnn_memory, detach_embedding,
+                                                         embedded=embedded)
         return value, emb, rnn_memory, full
+
+    def embed(self, state, lst_state, lst_action, rnn_memory: Optional[RNNHidden], reward):
+        """The context-encoder half of forward(): (embedding, its hidden, its per-layer record)."""
+        return self._meta_forward_embedding(self.get_embedding_input(state, lst_state, lst_action, reward), rnn_memory)
 
     def forward_embedding(self, state, lst_state, lst_action, rnn_memory, reward):
         return self.get_embedding(self.get_embedding_input(state, lst_state, lst_action, reward), rnn_memory)
