@@ -235,6 +235,7 @@ class FullLengthRNNUpdate:
             self.parameter.no_alpha_auto_tune = True
             policy_args = dict(policy_args, sample_std=self.parameter.sample_std)
         self.policy_args, self.value_args = policy_args, value_args
+        self.max_trajectory_len = int(max_trajectory_len)
         assert self.parameter.value_net_num == 1
         for item in value_args['uni_model_layer_type']:
             assert item.startswith('e')
@@ -375,6 +376,30 @@ class FullLengthRNNUpdate:
         if value_sd is not None:
             self.values[0].load_state_dict(value_sd)
         self._finalize_models()
+
+    def state_dict(self) -> dict:
+        """Everything a run needs to continue bit for bit where it stopped (algorithm/checkpoint.py, DESIGN.md §3.14):
+        weights of the four models under the reference's keys (the `policy` / `value` entries load with `load_models`),
+        Adam moments / step counts / frozen sets and the arena layouts, log-alpha, the Q guard, the cadence counters, the
+        cgpt dropout counters and salts, the replay buffer, and the numpy / torch CPU / CUDA random states, plus the
+        hyper-parameters and a structural signature.  Tensors on the CPU, ints, floats, bools and strings only: persist
+        it with `torch.save` and read it back with `torch.load(path, weights_only=True)`.  Rank-local under data
+        parallelism: every rank saves its own."""
+        from .checkpoint import state_dict
+        return state_dict(self)
+
+    def load_state_dict(self, sd: dict) -> None:
+        """Restore a `state_dict()` into this engine, in place: weights, moments, guard, alpha and counters are copied
+        into the tensors the engine already owns, so captured CUDA graphs stay valid unless something they bake in
+        (frozen-parameter segments, dropout salts) changed, in which case they are dropped.  The checkpoint is checked
+        before anything is touched: a different `format`, algorithm, encoder, width, ensemble size, action type, buffer
+        layout or arena layout raises ValueError naming the first differing field and leaves the engine as it was.
+        Hyper-parameters are not applied: the live engine's values are used.
+
+        Side effect: the process-global numpy and torch (CPU and this device's CUDA) random states are set to the
+        checkpoint's, because the replay sampler, the REDQ subset and the policy noise draw from them."""
+        from .checkpoint import load_state_dict
+        load_state_dict(self, sd)
 
     def _get_skip_len(self):
         """1 + widest causal-conv window of any encoder layer (ref: sac_full_length_rnn_ensembleQ.py:57-68)."""

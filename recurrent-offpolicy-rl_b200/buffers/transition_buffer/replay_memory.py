@@ -35,6 +35,34 @@ def _width(item) -> int:
     raise NotImplementedError(f'not implement for type of {type(item)}')
 
 
+def _encode_pending(memory: List[Transition]) -> dict:
+    """The partial trajectory `mem_push` collects until `done`, one float64 tensor per field stacked over the steps.
+    Fields given as Python / numpy scalars come back as Python floats, arrays and lists as float64 arrays: either way
+    they land in the buffer as the same float64 row."""
+    out = {'steps': len(memory)}
+    for i, name in enumerate(tuplenames):
+        vals = [t[i] for t in memory]
+        if all(v is None for v in vals):
+            continue
+        if any(v is None for v in vals):
+            raise ValueError(f'pending trajectory: field {name} is None in some steps only')
+        out[name] = torch.from_numpy(np.stack([np.asarray(v, dtype=np.float64) for v in vals]))
+        out[name + '.scalar'] = all(np.isscalar(v) for v in vals)
+    return out
+
+
+def _decode_pending(sd: dict) -> List[Transition]:
+    fields = []
+    for name in tuplenames:
+        if name not in sd:
+            fields.append([None] * sd['steps'])
+        elif sd[name + '.scalar']:
+            fields.append([float(x) for x in sd[name].tolist()])
+        else:
+            fields.append(list(sd[name].numpy()))
+    return [Transition(*[f[t] for f in fields]) for t in range(sd['steps'])]
+
+
 class MemoryArray(object):
     def __init__(self, max_transition_num: int = 1000000, max_traj_step: Optional[int] = 1000, rnn_slice_length=1,
                  device: Optional[torch.device] = None):
@@ -150,6 +178,53 @@ class MemoryArray(object):
                         self.complete_traj([Transition(*[f[i] if (f is not None and not np.isscalar(f)) else f for f in t])
                                             for t in self.memory])
             self.memory = []
+
+    # ---- checkpoint state ---------------------------------------------------------------------------------------
+    def column_widths(self) -> List[int]:
+        """Columns per `Transition` field, in field order ([] before the first trajectory fixes the layout)."""
+        return [len(r) for r in self.ind_range] if self.ind_range is not None else []
+
+    def state_dict(self) -> dict:
+        """Everything that decides what the buffer holds and what the sampler draws from it, as tensors / ints / strings
+        (`torch.load(weights_only=True)` reads it back): the host rows up to the end of the highest live trajectory (rows
+        above it are never read), the trajectory start / length lists, the write pointer, the transition count and the
+        pending partial trajectory.  The device mirror is not stored: it is the fp32 cast of the host rows."""
+        end = max((s + n for s, n in zip(self.trajectory_start, self.trajectory_length)), default=0)
+        rows = self.memory_buffer[:end] if self.memory_buffer is not None else np.zeros((0, 0))
+        return {'max_transition_num': self.max_transition_num, 'max_traj_step': int(self.max_traj_step),
+                'columns': self.column_widths(), 'rows': torch.from_numpy(np.array(rows, dtype=np.float64)),
+                'trajectory_start': torch.tensor(self.trajectory_start, dtype=torch.int64),
+                'trajectory_length': torch.tensor(self.trajectory_length, dtype=torch.int64),
+                'ptr': int(self.ptr), 'transition_count': int(self.transition_count), 'pending': _encode_pending(self.memory)}
+
+    def state_mismatch(self, sd: dict) -> Optional[str]:
+        """Name of the first structural field in which `sd` differs from this buffer, or None.  A buffer that has not seen
+        a trajectory yet takes any column layout."""
+        for k in ('max_transition_num', 'max_traj_step'):
+            if int(sd[k]) != int(getattr(self, k)):
+                return f'replay_buffer.{k}'
+        if sd['columns'] and self.ind_range is not None and list(sd['columns']) != self.column_widths():
+            return 'replay_buffer.columns'
+        return None
+
+    def load_state_dict(self, sd: dict) -> None:
+        """Restore what `state_dict()` saved.  The host and device buffers are kept (allocated from the saved column
+        layout if this buffer has none yet); the device rows are rewritten from the host rows with one copy."""
+        bad = self.state_mismatch(sd)
+        if bad is not None:
+            raise ValueError(f'replay-buffer state does not match this buffer: {bad}')
+        if sd['columns'] and self.memory_buffer is None:
+            self._init_memory_buffer(Transition(*[np.zeros(w) if w else None for w in sd['columns']]))
+        rows = sd['rows'].numpy()
+        end = rows.shape[0]
+        if end:
+            self.memory_buffer[:end] = rows
+            if self.device_buffer is not None:
+                self.device_buffer[:end].copy_(torch.from_numpy(rows.astype(np.float32)))
+        self.trajectory_start = [int(x) for x in sd['trajectory_start'].tolist()]
+        self.trajectory_length = [int(x) for x in sd['trajectory_length'].tolist()]
+        self.ptr, self.transition_count = int(sd['ptr']), int(sd['transition_count'])
+        self.memory = _decode_pending(sd['pending'])
 
     # ---- trajectory index draw (numpy global RNG; call order is part of the parity contract) ----------------
     def _traj_ind_sample(self, batch_size, max_sample_size) -> np.ndarray:
