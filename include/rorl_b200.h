@@ -472,6 +472,35 @@ int rorl_skinny_wgrad(const float* g, const float* x, float* dW, float* work, in
                       int64_t ldg, int64_t ldx, int64_t seg_rows, int64_t seg_stride, cudaStream_t stream);
 int rorl_skinny_dgrad(const float* g, const float* W, float* dx, int64_t M, int64_t N, int64_t K, int64_t ldg, cudaStream_t stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Decode step (csrc/step.cu): what one environment step of the policy (L = 1) runs.
+ *
+ * rorl_small_linear: y[g][m, n] = act(bias[g][n] + sum_k x[g][m, k] W[g](n, k)) for 1 <= M <= 64 rows, any K >= 1, any N,
+ * in fp32 on the FMA pipe (the rollout's projections; a tensor-core tile would compute one to a few real rows).
+ *   layout 0: W [N, K] (nn.Linear), G = 1, x_gstride = 0, bias [N];
+ *   layout 1: W [G, K, N] (EnsembleLinear), bias [G, N]; x of member g at x + g * x_gstride (0 = one input shared by
+ *             all G members); y of member g at y + g * M * ldy.
+ * Row m of x is at x + m * ldx (ldx >= K), row m of y at y + m * ldy (ldy >= N).  bias may be NULL; elu != 0 applies ELU.
+ * The summation order along K is fixed by the block shape, not the grid: repeated calls are bit-identical.
+ *
+ * rorl_mamba_step_conv: one step of the smamba mixer's depthwise conv (ref: smamba/mamba.py Mamba.step): the window
+ * [B, D, Kc] (row b at win + b * ld_win) is rolled left by one and the new column xs = xz[b, :D] appended, then
+ * u[b, d] = silu(sum_j window[b, d, j] conv_w[d, j] + conv_b[d]) into u [B, D] contiguous.  conv_b may be NULL.
+ * rorl_mamba_step_ssm: one step of the selective SSM with the carried state h [B, D, Ns] (row b at h + b * ld_h):
+ *   delta = softplus(x_dbl[b, :R] . dt_w[d, :] + dt_b[d]);  A = -exp(A_log[d, n]);
+ *   h <- exp(delta A) h + delta u B (B = x_dbl[b, R:R+Ns]);  y[b, d] = (C . h + Dskip[d] u) silu(z[b, d])
+ * with C = x_dbl[b, R+Ns:R+2Ns]; y [B, D] contiguous; Dskip may be NULL.  For both, win_in / h_in may equal win_out /
+ * h_out (update in place).  As in the reference's step, no reset flag or mask is read.
+ * ---------------------------------------------------------------------------------------------- */
+int rorl_small_linear(const float* x, int64_t ldx, int64_t x_gstride, const float* W, const float* bias, float* y, int64_t ldy,
+                      int64_t M, int64_t N, int64_t K, int64_t G, int layout, int elu, cudaStream_t stream);
+int rorl_mamba_step_conv(const float* xz, int64_t ld_xz, const float* conv_w, const float* conv_b, const float* win_in,
+                         int64_t ld_win_in, float* win_out, int64_t ld_win_out, float* u, int64_t B, int64_t D, int64_t Kc,
+                         cudaStream_t stream);
+int rorl_mamba_step_ssm(const float* u, const float* x_dbl, int64_t ld_xdbl, const float* z, int64_t ld_z, const float* dt_w,
+                        const float* dt_b, const float* A_log, const float* Dskip, const float* h_in, int64_t ld_h_in, float* h_out,
+                        int64_t ld_h_out, float* y, int64_t B, int64_t D, int64_t R, int64_t Ns, cudaStream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -20,7 +20,7 @@ HEADER = os.path.join(REPO_ROOT, "include", "rorl_b200.h")
 LIB_PATH = os.environ.get("RORL_B200_LIB") or os.path.join(CSRC, "librorl_b200.so")   # override: A/B experiments only
 SOURCES = ["scan_real.cu", "scan_complex.cu", "selscan.cu", "conv1d.cu", "addnorm.cu", "losses.cu", "optim.cu",
            "gather.cu", "gru.cu", "lstm.cu", "gemm_bf16.cu", "attn.cu", "reduce.cu", "efc_head.cu", "head.cu",
-           "categorical.cu"]
+           "categorical.cu", "step.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v"]
 

@@ -278,6 +278,7 @@ class FullLengthRNNUpdate:
     def _finalize_models(self):
         """(Re)build arenas + optimizers after weights are in place; call again after load_state_dict."""
         self._graphs, self._graph_pool = {}, None       # captured graphs point into the old arenas
+        self.model_generation = getattr(self, 'model_generation', -1) + 1     # actors (make_actor) recapture on a change
         for m in [self.policy, self.target_policy] + list(self.values) + list(self.target_values):
             m.need_full_hidden = False                  # the update never reads forward()'s per-layer output record
         gpt = any(str(t).startswith(('cgpt', 'gpt', 'transformer')) for m in (self.policy, self.values[0])
@@ -369,6 +370,14 @@ class FullLengthRNNUpdate:
         on a live object; weights, optimizer state and learning-rate tables live in device memory and need no
         re-capture.  (`load_models` / `_finalize_models` call it themselves: the arenas move.)"""
         self._graphs, self._graph_pool = {}, None
+
+    def make_actor(self, n_envs: int, use_cuda_graph: Optional[bool] = None):
+        """A `PolicyActor` (algorithm/actor.py) that acts for `n_envs` environments stepped in lockstep: per step one
+        pinned H2D copy, one CUDA-graph replay of `policy.forward` at L = 1 with every layer's hidden state carried on
+        the device, one D2H copy.  Rank-local under data parallelism.  Not available for the cgpt encoder."""
+        from .actor import PolicyActor
+        graph = self.use_cuda_graph if use_cuda_graph is None else use_cuda_graph
+        return PolicyActor(self.policy, n_envs, generation=lambda: self.model_generation, use_cuda_graph=graph)
 
     def load_models(self, policy_sd=None, value_sd=None):
         if policy_sd is not None:

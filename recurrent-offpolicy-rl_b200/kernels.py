@@ -1099,11 +1099,95 @@ def linear_gelu(x, weight, bias=None, passes=2):
     return LinearTC.apply(x, weight, bias, 2, passes)
 
 
+# ------------------------------------------------------------------------------------------------
+# decode step (csrc/step.cu): the policy acting for a batch of environments, L = 1
+# ------------------------------------------------------------------------------------------------
+SMALL_LINEAR_MAX_ROWS = 64
+# False restores the tensor-core / cuBLAS / torch path for decode-step shapes too (A/B timing in tools/bench_act.py)
+DECODE_STEP_KERNELS = True
+
+
+def decode_step_ok(x: torch.Tensor, rows: int, *params) -> bool:
+    """Is this call one rollout step the decode kernels take?  x [.., 1, K] (time axis 1) on CUDA in fp32, at most
+    SMALL_LINEAR_MAX_ROWS rows, and autograd not recording it (no gradient flows through the decode kernels).  Every
+    update input has L >= 2, so no call inside an update qualifies."""
+    if not (DECODE_STEP_KERNELS and x.is_cuda and x.dtype == torch.float32 and x.dim() >= 3 and x.shape[-2] == 1
+            and 1 <= rows <= SMALL_LINEAR_MAX_ROWS):
+        return False
+    return not (torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (x, *params)))
+
+
+def _rows2d(x: torch.Tensor, K: int):
+    """[.., K] -> ([M, K] view with unit inner stride, row stride) (a copy only if no such view exists)."""
+    x2 = x.reshape(-1, K)
+    if x2.stride(-1) != 1:
+        x2 = x2.contiguous()
+    return x2, (x2.stride(0) if x2.shape[0] > 1 else K)
+
+
+def small_linear(x, weight, bias=None, elu=False, layout=0, shared=True, out=None):
+    """rorl_small_linear.  layout 0: x [M, K] (any row stride), weight [N, K], bias [N] -> [M, N].
+    layout 1: weight [G, K, N], bias [G, N] (or [G, 1, N]); x [M, K] shared by the G members, or [G, M, K] with
+    shared=False -> [G, M, N].  M <= 64.  out: a [M, N] destination with unit inner stride (layout 0 only)."""
+    if layout == 0:
+        Nn, K = weight.shape
+        G = 1
+    else:
+        G, K, Nn = weight.shape
+    if shared:
+        x2, ldx = _rows2d(x, K)
+        xg = 0
+    else:
+        x3 = x.reshape(G, -1, K)
+        if x3.stride(-1) != 1 or (x3.shape[1] > 1 and x3.stride(1) < K):
+            x3 = x3.contiguous()
+        x2, ldx, xg = x3, (x3.stride(1) if x3.shape[1] > 1 else K), x3.stride(0)
+    M = x2.shape[-2]
+    w = _f32c(weight)
+    b = None if bias is None else _f32c(bias.reshape(-1))
+    if out is not None:
+        assert layout == 0 and tuple(out.shape) == (M, Nn) and out.stride(-1) == 1 and out.dtype == torch.float32
+        y, ldy = out, (out.stride(0) if M > 1 else Nn)
+    else:
+        y = torch.empty((M, Nn) if layout == 0 else (G, M, Nn), device=x.device, dtype=torch.float32)
+        ldy = Nn
+    N.call("rorl_small_linear", N.ptr(x2), ldx, xg, N.ptr(w), N.ptr(b), N.ptr(y), ldy, M, Nn, K, G, int(layout), int(bool(elu)),
+           N.stream())
+    return y
+
+
+def mamba_step_conv(xz, conv_w, conv_b, win_in, win_out, Dn):
+    """Roll the [B, Dn, Kc] conv window (row-strided views of the carried hidden), append xz[:, :Dn] and return
+    u = silu(depthwise conv + bias) [B, Dn].  win_in may be win_out (in place)."""
+    B = xz.shape[0]
+    Kc = conv_w.shape[-1]
+    u = torch.empty((B, Dn), device=xz.device, dtype=torch.float32)
+    N.call("rorl_mamba_step_conv", N.ptr(xz), xz.stride(0), N.ptr(_f32c(conv_w.reshape(Dn, Kc))),
+           N.ptr(None if conv_b is None else _f32c(conv_b)), N.ptr(win_in), win_in.stride(0), N.ptr(win_out), win_out.stride(0),
+           N.ptr(u), B, Dn, Kc, N.stream())
+    return u
+
+
+def mamba_step_ssm(u, x_dbl, z, dt_w, dt_b, A_log, Dskip, h_in, h_out):
+    """One selective-SSM step with the carried state (row-strided [B, Dn * Ns] views; h_in may be h_out): advances h and
+    returns y [B, Dn] = (C . h + D u) silu(z).  x_dbl [B, R + 2 Ns], z [B, Dn] with unit inner strides."""
+    B, Dn = u.shape
+    R, Ns = dt_w.shape[1], A_log.shape[1]
+    y = torch.empty((B, Dn), device=u.device, dtype=torch.float32)
+    N.call("rorl_mamba_step_ssm", N.ptr(u), N.ptr(x_dbl), x_dbl.stride(0), N.ptr(z), z.stride(0), N.ptr(_f32c(dt_w)), N.ptr(_f32c(dt_b)),
+           N.ptr(_f32c(A_log)), N.ptr(None if Dskip is None else _f32c(Dskip)), N.ptr(h_in), h_in.stride(0), N.ptr(h_out),
+           h_out.stride(0), N.ptr(y), B, Dn, R, Ns, N.stream())
+    return y
+
+
 def linear(x, weight, bias=None, elu=False, passes=2):
     """nn.Linear forward (+ optional fused ELU).  Shapes the tensor-core kernel cannot take (K % 4, N % 4, K < 32)
     go through cuBLAS; both are GPU paths.  passes=4: one bf16 MMA per product (used where the reference itself runs
-    the layer in bf16 autocast), default 2 = two-term bf16 split, fp32 parity."""
+    the layer in bf16 autocast), default 2 = two-term bf16 split, fp32 parity.  A decode-step call (decode_step_ok,
+    passes == 2) runs on rorl_small_linear."""
     M = x.numel() // x.shape[-1]
+    if passes == 2 and decode_step_ok(x, M, weight, bias):
+        return small_linear(x, weight, bias, elu).view(*x.shape[:-1], weight.shape[0])
     if x.is_cuda and _gemm_ok(M, weight.shape[0], weight.shape[1]):
         return LinearTC.apply(x, weight, bias, elu, passes)
     if x.is_cuda and weight.shape[1] <= 16 and M >= 1024 and x.dtype == torch.float32:
@@ -1202,6 +1286,9 @@ def ensemble_hidden_to_scalar_ok(x, W2, W3):
 def ensemble_linear(x, weight, bias, elu, shared):
     E, Kin, Nout = weight.shape
     M = x.numel() // Kin // (1 if shared else E)
+    if decode_step_ok(x, M, weight, bias):
+        lead = x.shape[:-1] if shared else x.shape[1:-1]
+        return small_linear(x, weight, bias, elu, layout=1, shared=shared).view(E, *lead, Nout)
     if x.is_cuda and _gemm_ok(M, Nout, Kin):
         return EnsembleLinearTC.apply(x, weight, bias, elu, shared)
     return None

@@ -111,6 +111,8 @@ class Mamba(nn.Module):
         at on this path (SURVEY.md App. G)."""
         Bsz = x.shape[0]
         Dn, N, R, Kc = self.d_inner, self.d_state, self.dt_rank, self.d_conv
+        if self.use_conv and K.decode_step_ok(x, Bsz, *self.parameters()):
+            return self._step_fused(x, hidden)
         if hidden is None:
             conv_state = x.new_zeros((Bsz, Dn, Kc)) if self.use_conv else None
             ssm_state = x.new_zeros((Bsz, Dn, N))
@@ -132,6 +134,24 @@ class Mamba(nn.Module):
         out = self.out_proj(y)
         parts = ([conv_state.reshape(1, Bsz, -1)] if self.use_conv else []) + [last.reshape(1, Bsz, -1)]
         return out, torch.cat(parts, dim=-1)
+
+    def _step_fused(self, x, hidden):
+        """The same step on the decode kernels (csrc/step.cu): in_proj, x_proj and out_proj on rorl_small_linear, the
+        window roll + conv + SiLU in one kernel, dt_proj + softplus + the state update + D skip + SiLU(z) gate in
+        another.  The new [conv window | SSM state] is written to a fresh [1, B, .] tensor; `hidden` is only read."""
+        Bsz = x.shape[0]
+        Dn = self.d_inner
+        new = torch.empty((1, Bsz, self.desired_hidden_dim), device=x.device, dtype=torch.float32)
+        if hidden is None:
+            hidden = torch.zeros_like(new)
+        h_in, h_out = hidden[0], new[0]                                 # [B, conv | ssm], row-strided
+        cd = self.conv_hidden_dim
+        xz = self.in_proj(x).view(Bsz, 2 * Dn)                         # [B, 2D]: xs | z
+        u = K.mamba_step_conv(xz, self.conv1d.weight, self.conv1d.bias, h_in[:, :cd], h_out[:, :cd], Dn)
+        x_dbl = self.x_proj(u.view(Bsz, 1, Dn)).view(Bsz, -1)           # [B, R + 2N]
+        y = K.mamba_step_ssm(u, x_dbl, xz[:, Dn:], self.dt_proj.weight, self.dt_proj.bias, self.A_log, self.D,
+                             h_in[:, cd:], h_out[:, cd:])
+        return self.out_proj(y.view(Bsz, 1, Dn)), new
 
 
 def _init_weights(module, n_layer, rescale_prenorm_residual=True, n_residuals_per_layer=1):
